@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload rosenbrock|quadratic|driver3_f32] [--scaling auto|strong|weak] [--n N] [--m M]
+                    [--dump-outputs DIR]
 
 A "step" is one L-BFGS-B iteration: one pass of mainlb's main loop ending in 'NEW_X'
 (src/lbfgsb.f90:599-872) plus the caller's f/g evaluations for it (a device kernel inside the timed region).
@@ -30,7 +31,15 @@ real64, factr = pgtol = 0 and a fixed iteration budget.
 
 Warm-up: the driver's --warmup is raised to m + 4 iterations (history full, col = m) and extended (up to 10 more)
 until fewer than n/100 variables enter or leave the free set; `warmup` echoes the flag, `warmup_effective` says
-what ran.  --impl reference times the CPU port of the reference on the same workload (N = 1: the full n).
+what ran.  The headline times exactly --steps iterations (default 20; 12 for the quadratic, which converges after
+about 34 iterations); a solve that ends before them is an error.
+--impl reference times the CPU port of the reference on the same workload (N = 1: the full n).
+
+--dump-outputs DIR writes what the headline's last timed iteration left in the caller's hands: DIR/x.npy and DIR/g.npy
+(the iterate and its gradient, in the workload's dtype, at the global indices of DIR/index.npy: every variable up to
+2^20 of them, else one variable at a hashed position in each of 2^20 equal stretches, fixed by integer arithmetic
+alone) and DIR/f.npy.  The inputs depend on the arguments only, so two builds run with the same arguments can be
+compared file for file.
 """
 import argparse
 import json
@@ -51,19 +60,21 @@ METRIC = "lbfgsb_iterations_per_s"
 UNIT = "iterations/s"
 QUAD_SEED = 0
 QUAD_SCALE = 0.5
+DUMP_SAMPLE = 1 << 20   # --dump-outputs: x, g and index at 8 bytes each come to 24 MiB
+DUMP_SEED = 2024
 
-# BASELINE.json configs: name -> (n per single-GPU problem, m, numpy dtype name, odd lower bound)
+# BASELINE.json configs: name -> (n per single-GPU problem, m, numpy dtype name, odd lower bound, default --steps)
 WORKLOADS = {
-    "rosenbrock": dict(n=100_000_000, m=10, dtype="float64", l_odd=L_ODD, config="configs[2]"),
-    "quadratic": dict(n=125_000_000, m=10, dtype="float64", l_odd=None, config="configs[3]"),
-    "driver3_f32": dict(n=400_000_000, m=20, dtype="float32", l_odd=1.0, config="configs[4]"),
+    "rosenbrock": dict(n=100_000_000, m=10, dtype="float64", l_odd=L_ODD, config="configs[2]", steps=20),
+    "quadratic": dict(n=125_000_000, m=10, dtype="float64", l_odd=None, config="configs[3]", steps=12),
+    "driver3_f32": dict(n=400_000_000, m=20, dtype="float32", l_odd=1.0, config="configs[4]", steps=20),
 }
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20, help="timed iterations")
+    ap.add_argument("--steps", type=int, default=None, help="timed iterations (default: the workload's, see the header)")
     ap.add_argument("--warmup", type=int, default=14, help="untimed iterations (raised to m + 4, see the header)")
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--workload", default="rosenbrock", choices=sorted(WORKLOADS))
@@ -79,8 +90,16 @@ def parse():
     ap.add_argument("--ref-budget-s", type=float, default=float(os.environ.get("LBFGSB_REF_BUDGET_S", "480")),
                     help="--impl reference: stop timing early when the run has taken this long")
     ap.add_argument("--profile-out", default=None, help="write the per-kernel-family table here (JSON)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write x, g (sampled, see the header) and f of the last timed iteration as DIR/<name>.npy")
     a = ap.parse_args()
     wl = WORKLOADS[a.workload]
+    if a.steps is None:
+        a.steps = wl["steps"]
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     if a.n is None:
         a.n = wl["n"]
     if a.m is None:
@@ -133,6 +152,36 @@ def effective_warmup(W, m):
 
 def is_burst(nseg, nenter, nleave, n_global):
     return nseg > 1 or (nenter + nleave) > n_global // 100
+
+
+def dump_index(n_global, size=None):
+    """Global indices of the variables --dump-outputs writes (default size DUMP_SAMPLE): all of them up to `size`, else
+    one in each of `size` equal stretches, at a position given by the splitmix64 hash of the stretch number and
+    DUMP_SEED.  Sorted, and the same in every run, on every rank and with every numpy version (no random stream)."""
+    size = DUMP_SAMPLE if size is None else int(size)
+    if n_global <= size:
+        return np.arange(n_global, dtype=np.int64)
+    k = np.arange(size + 1, dtype=np.int64)
+    edge = k * n_global // size
+    z = (k[:-1] + DUMP_SEED + 1).astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15)   # integer ops wrap mod 2^64
+    z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+    z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+    z ^= z >> np.uint64(31)
+    return edge[:-1] + (z % np.diff(edge).astype(np.uint64)).astype(np.int64)
+
+
+def shard_positions(idx, lo, hi):
+    """(positions in idx, local indices) of the global indices idx that lie in the shard [lo, hi)."""
+    mine = (idx >= lo) & (idx < hi)
+    return np.flatnonzero(mine), idx[mine] - lo
+
+
+def write_outputs(path, outputs):
+    """outputs: name -> float32 / float64 array, written as path/<name>.npy."""
+    os.makedirs(path, exist_ok=True)
+    for name, v in outputs.items():
+        assert v.dtype in (np.float32, np.float64), (name, v.dtype)
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -464,6 +513,24 @@ class DeviceSolve:
         return dict(iter=int(p.isave[29]), nseg=int(p.isave[32]), nfree=int(p.isave[37]), nenter=int(p.isave[40]),
                     nleave=int(self.n_global + 1 - p.isave[39]), col=int(p.isave[27]), nfgv=int(p.isave[33]))
 
+    def outputs(self):
+        """x and g at dump_index(n_global), f, and the indices (as float64), as the solve stands; every rank of a
+        sharded solve returns all of them."""
+        torch, dev = self.cx.torch, self.cx.dev
+        idx = dump_index(self.n_global)
+        dst, src = (torch.from_numpy(a).to(dev) for a in shard_positions(idx, self.off, self.off + self.n))
+        out = {}
+        for name in ("x", "g"):
+            v = getattr(self, name)
+            s = torch.zeros(idx.size, dtype=v.dtype, device=dev)
+            s[dst] = v[src]
+            if self.world > 1:
+                self.cx.dist.all_reduce(s)   # each index lies in one shard: the other ranks add zeros
+            out[name] = s.cpu().numpy()
+        out["f"] = self.prob.f.copy()
+        out["index"] = idx.astype(np.float64)
+        return out
+
     def close(self):
         self.prob.close()
         for k in ("x", "l", "u", "nbd", "g"):
@@ -471,9 +538,11 @@ class DeviceSolve:
         self.cx.torch.cuda.empty_cache()
 
 
-def measure(cx, kind, n_global, m, dtype, l_odd, W, K, plain_fg=False, sharded_run=None, profile_k=None, want_clocks=True):
+def measure(cx, kind, n_global, m, dtype, l_odd, W, K, plain_fg=False, sharded_run=None, profile_k=None, want_clocks=True,
+            want_outputs=False):
     """Warm-up, K timed iterations (CUDA events per iteration on the engine's stream), per-kernel-family pass.
-    Returns the result dict of this workload (rank-independent fields are identical on every rank)."""
+    Returns the result dict of this workload (rank-independent fields are identical on every rank); with want_outputs,
+    its "outputs" are DeviceSolve.outputs() after the last timed iteration."""
     torch = cx.torch
     ds = DeviceSolve(cx, kind, n_global, m, dtype, l_odd, plain_fg, sharded_run)
     prob = ds.prob
@@ -512,10 +581,12 @@ def measure(cx, kind, n_global, m, dtype, l_odd, W, K, plain_fg=False, sharded_r
         if clocks:
             clocks.stop_flag = True
         if not ok or len(rows) != K:
-            raise SystemExit("solve ended inside the timed region: " + prob.task_str())
+            raise SystemExit("solve ended inside the timed region after %d of %d steps: %s" % (len(rows), K, prob.task_str()))
         ms = cx.max_over_ranks(evs[0].elapsed_time(evs[K]))
         per = [evs[i].elapsed_time(evs[i + 1]) for i in range(K)]
         l1, s1 = prob.counters()
+        if want_outputs:
+            out["outputs"] = ds.outputs()
         fg_evals = ds.nfg - f0
         # our kernels per objective evaluation: the objective kernel + its final sum (+ 4 exchange kernels on a shard)
         fg_kernels = 2 if ds.world == 1 else 6
@@ -718,13 +789,15 @@ def main():
     n_global = a.n if strong else a.n * world
     n_local = -(-n_global // world)
     W, K = a.warmup, a.steps
-    Kh = K if a.workload != "quadratic" else min(K, 12)   # the quadratic reaches machine precision after ~34 iterations
 
-    head = measure(cx, a.workload, n_global, a.m, dtype, l_odd, W, Kh, a.plain_fg)
+    head = measure(cx, a.workload, n_global, a.m, dtype, l_odd, W, K, a.plain_fg, want_outputs=bool(a.dump_outputs))
+    outputs = head.pop("outputs", None)
+    if outputs is not None and rank == 0:
+        write_outputs(a.dump_outputs, outputs)
     cfg = base_config(a.workload, n_global, n_local, a.m, world, ("strong" if strong else "weak") if world > 1 else "single",
                       dtype, l_odd)
     out = {
-        "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world, "steps": Kh, "warmup": W,
+        "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
         "warmup_effective": head["warmup_effective"], "ms_per_step": head["ms_per_step"], "higher_is_better": True,
         "scaling": "strong" if strong else "weak", "vs_baseline": None,
         "dtype": "f64" if np.dtype(dtype) == np.float64 else "f32", "data": "synthetic", "config": cfg,
@@ -787,7 +860,7 @@ def main():
     # ---- e2e: HOST buffers ----
     if not a.no_e2e:
         try:
-            out["e2e"] = e2e_host(cx, a.workload, n_global, a.m, W, Kh, l_odd)
+            out["e2e"] = e2e_host(cx, a.workload, n_global, a.m, W, K, l_odd)
         except Exception as e:  # noqa: BLE001
             out["e2e"] = {"value": None, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0,
                           "note": "failed: %s: %s" % (type(e).__name__, e)}
