@@ -140,7 +140,9 @@ void lbfgsb_dev_nccl_destroy(void* comm);
 int lbfgsb_dev_active_set_hash(lbfgsb_dev_t* h, uint64_t* hash, int64_t* count);
 /* device pointer of a work vector: 0 z, 1 r, 2 d, 3 t, 4 xp, 5 ws, 6 wy, 7 iwhere, 8 previous gradient */
 void* lbfgsb_dev_vector(lbfgsb_dev_t* h, int32_t which);
-/* device-to-device copy of `bytes` bytes of that work vector into dst_dev (after the engine's stream drained) */
+/* device-to-device copy of `bytes` bytes of that work vector into dst_dev (after the engine's stream drained); returns 1
+   without copying when `bytes` exceeds the vector's allocation: m * ldw reals for 5 and 6 (ldw = n rounded up to a
+   multiple of 32), ldw int32 for 7, ldw reals otherwise */
 int lbfgsb_dev_vector_copy(lbfgsb_dev_t* h, int32_t which, void* dst_dev, int64_t bytes);
 /* how the per-rank reduction records travel on a sharded workspace: 0 single GPU, 1 ncclAllGather, 2 stores into the
  * peers' memory over NVLink (CUDA IPC; default when every rank can map every peer, LBFGSB_B200_P2P=0 switches it off) */

@@ -398,7 +398,9 @@ class DeviceProblem:
         return out
 
     def vector(self, which, count=None, dtype=None):
-        """Copy of a work vector: 0 z, 1 r, 2 d, 3 t, 4 xp, 7 iwhere (diagnostics)."""
+        """Copy of a work vector (diagnostics): 0 z, 1 r, 2 d, 3 t, 4 xp, 7 iwhere, 8 the previous gradient, all of n
+        elements by default; 5 ws and 6 wy hold m columns of ldw = roundup(n, 32) reals (column j of the S/Y ring at
+        j * ldw), so pass count = m * ldw for them.  A count beyond the vector's allocation raises."""
         torch = self.torch
         n = self.n if count is None else count
         tdt = {np.dtype(np.float64): torch.float64, np.dtype(np.float32): torch.float32}[self.dtype]

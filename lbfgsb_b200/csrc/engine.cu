@@ -2376,6 +2376,12 @@ void* lbfgsb_dev_vector(lbfgsb_dev_t* h, int32_t which) {
 int lbfgsb_dev_vector_copy(lbfgsb_dev_t* h, int32_t which, void* dst_dev, int64_t bytes) {
     void* src = lbfgsb_dev_vector(h, which);
     if (!src || !dst_dev || bytes < 0) return 1;
+    // never copy past the vector's allocation: m columns of ldw reals for ws / wy, ldw int32 for iwhere, ldw reals else
+    EngineBase* b = (EngineBase*)h;
+    const i64 ldw = (b->real_kind == 8) ? ((Engine<double>*)b)->w.ldw : ((Engine<float>*)b)->w.ldw;
+    const i64 m = (b->real_kind == 8) ? ((Engine<double>*)b)->w.m : ((Engine<float>*)b)->w.m;
+    const i64 cap = (which == 7) ? ldw * 4 : ((which == 5 || which == 6) ? m : 1) * ldw * (i64)b->real_kind;
+    if (bytes > cap) { set_error("lbfgsb_dev_vector_copy: %lld bytes requested, vector %d holds %lld", (long long)bytes, (int)which, (long long)cap); return 1; }
     if (cudaDeviceSynchronize() != cudaSuccess) return 1;
     return cudaMemcpy(dst_dev, src, (size_t)bytes, cudaMemcpyDeviceToDevice) != cudaSuccess;
 }

@@ -1609,6 +1609,7 @@ struct LB {
                            col, head, wa, wa + 2 * m, wa + 4 * m, wa + 6 * m, nseg_l, sbgnrm, info,
                            epsmch);
                     if (info != 0) {
+                        g_events[2]++;  // refresh the lbfgs memory and restart the iteration
                         info = 0;
                         col = 0;
                         head = 1;
@@ -1636,6 +1637,7 @@ struct LB {
                         formk(n, nfree, index, nenter, ileave, indx2, iupdat, updatd, wn, snd, m, ws,
                               wy, sy, theta, col, head, info);
                     if (info != 0) {
+                        g_events[2]++;  // refresh the lbfgs memory and restart the iteration
                         info = 0;
                         col = 0;
                         head = 1;
@@ -1655,6 +1657,7 @@ struct LB {
                               head, iword, wa, wn, info);
                     }
                     if (info != 0) {
+                        g_events[2]++;  // refresh the lbfgs memory and restart the iteration
                         info = 0;
                         col = 0;
                         head = 1;
@@ -1695,6 +1698,7 @@ struct LB {
                         return;
                     } else {
                         if (info == 0) nfgv = nfgv - 1;
+                        g_events[2]++;  // refresh the lbfgs memory and restart the iteration
                         info = 0;
                         col = 0;
                         head = 1;
@@ -1745,6 +1749,7 @@ struct LB {
                 ddum = -gdold * stp;
             }
             if (dr <= epsmch * ddum) {  // :826-834
+                g_events[3]++;
                 nskip = nskip + 1;
                 updatd = false;
                 prelims = true;
@@ -1756,6 +1761,7 @@ struct LB {
             matupd(n, m, ws, wy, sy, ss, d, r, itail, iupdat, col, head, theta, rr, dr, stp, dtd);
             formt(m, wt, sy, ss, col, theta, info);
             if (info != 0) {
+                g_events[2]++;  // refresh the lbfgs memory and restart the iteration
                 info = 0;
                 col = 0;
                 head = 1;

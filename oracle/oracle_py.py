@@ -89,7 +89,8 @@ def set_sum_mode(mode):
 
 
 def event_counts(reset=True):
-    """[subsm backtracks (:2830), ascent directions (:2247), ...] seen by the oracle since the last reset."""
+    """[subsm backtracks (:2830), ascent directions (:2247), memory resets ("refresh the lbfgs memory"), skipped
+    updates (:826-834), 0, 0, 0, 0] seen by the oracle since the last reset."""
     out = (C.c_longlong * 8)()
     lib().oracle_event_counts(out, C.c_int(1 if reset else 0))
     return list(out)

@@ -1,6 +1,6 @@
 """Edge cases of the iteration path against the oracle (same f/g routine on both sides): tiny n, m = 1, m > n,
-every variable fixed, start on the bounds, non-convex objectives that skip BFGS updates (:826-834) and reset the
-memory, and a seeded sweep over mixed bound kinds."""
+every variable fixed, start on the bounds, non-convex objectives that skip BFGS updates (:826-834) and backtrack in the line
+search, and a seeded sweep over mixed bound kinds."""
 import numpy as np
 import pytest
 
@@ -71,34 +71,44 @@ def test_all_variables_fixed_and_start_on_bounds():
     del lbfgsb_b200
 
 
-def _nonconvex(n, seed):
+def _nonconvex(n, seed, share, a_c):
+    """A box-constrained objective with a concave part: -a_c * a * x^2 on a share of the variables (the minimiser of
+    those lies on a bound), a * (x - b)^2 on the others, coupled by 1/4 sum (x[i+1] - x[i])^2.  Along a step into
+    the concave part s'y <= 0, and the update is skipped (:826-834)."""
     rng = np.random.default_rng(seed)
-    c = rng.uniform(0.5, 2.0, n)
+    conc = rng.random(n) < share
+    a = rng.uniform(0.5, 2.0, n)
+    b = rng.uniform(-1.0, 1.0, n)
 
     def fg(x, g):
-        s, co = np.sin(c * x), np.cos(c * x)
-        f = float(s.sum() + 0.1 * float((x[:-1] * x[1:]).sum()) + 0.01 * float((x ** 4).sum()))
-        g[:] = c * co + 0.04 * x ** 3
-        g[:-1] += 0.1 * x[1:]
-        g[1:] += 0.1 * x[:-1]
-        return f
-    return fg
-
-
-@pytest.mark.parametrize("n,m,seed", [(400, 5, 0), (3000, 10, 1), (20001, 7, 2)])
-def test_nonconvex_objective_with_skips_and_line_search_backtracks(n, m, seed):
-    fg = _nonconvex(n, seed)
+        r = x - b
+        t = x[1:] - x[:-1]
+        g[:] = np.where(conc, -2.0 * a_c * a * x, 2.0 * a * r)
+        g[1:] += 0.5 * t
+        g[:-1] -= 0.5 * t
+        return float(np.where(conc, -a_c * a * x * x, a * r * r).sum() + 0.25 * (t * t).sum())
 
     def mk():
-        rng = np.random.default_rng(100 + seed)
-        return rng.uniform(-3, 3, n), np.full(n, -3.0), np.full(n, 3.0), np.full(n, 2, np.int32)
+        r2 = np.random.default_rng(seed + 100)
+        return r2.uniform(-0.5, 0.5, n), np.full(n, -2.0), np.full(n, 2.0), np.full(n, 2, np.int32)
+    return fg, mk
+
+
+@pytest.mark.parametrize("n,m,seed,share,a_c", [(400, 5, 0, 0.5, 0.3), (3000, 10, 1, 0.3, 1.0), (20001, 7, 2, 0.1, 2.0)])
+def test_nonconvex_objective_with_skips_and_line_search_backtracks(n, m, seed, share, a_c):
+    fg, mk = _nonconvex(n, seed, share, a_c)
+    O.event_counts()
     gpu, ref = _both(fg, mk, n, m, factr=0.0, pgtol=0.0, budget=30)
+    ev = O.event_counts()
     _check(gpu, ref, upto=14)
-    assert any(r["iback"] > 0 for r in ref[0][:14]) or any(r["nskip"] > 0 for r in ref[0][:14]) or True
+    # the oracle skipped an update with pairs in the memory (col > 0) and backtracked in the line search
+    assert ev[3] >= 1, ev
+    assert any(b["nskip"] > a["nskip"] and a["col"] > 0 for a, b in zip(ref[0][:14], ref[0][1:14])), ref[0][:14]
+    assert any(r["iback"] > 0 for r in ref[0][:14])
 
 
-@pytest.mark.parametrize("seed", [11, 12, 13, 14, 15, 16])
-def test_seeded_sweep_mixed_bounds(seed):
+def sweep_problem(seed):
+    """(n, m, fg, mk) of a seeded mixed-bound problem: nbd in {0, 1, 2, 3}, 3 % fixed variables, a coupled quartic."""
     rng = np.random.default_rng(seed)
     n = int(rng.integers(60, 6000))
     m = int(rng.integers(1, 13))
@@ -124,5 +134,11 @@ def test_seeded_sweep_mixed_bounds(seed):
         u[fx] = l[fx]
         nbd[fx] = 2
         return x, l, u, nbd
+    return n, m, fg, mk
+
+
+@pytest.mark.parametrize("seed", [11, 12, 13, 14, 15, 16])
+def test_seeded_sweep_mixed_bounds(seed):
+    n, m, fg, mk = sweep_problem(seed)
     gpu, ref = _both(fg, mk, n, m, factr=1e3, pgtol=1e-8, budget=25)
     _check(gpu, ref, upto=10)

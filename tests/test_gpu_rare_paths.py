@@ -145,6 +145,7 @@ def test_ascent_direction_restart_withdraws_speculative_step_f32():
     for n, m, l_odd, x0 in F32_ASCENT_CASES:
         gpu, ref, ev, total = _run_pair(n, m, l_odd, x0, np.float32, 120)
         assert total[1] >= 1, ("the oracle met no ascent direction on this problem: the case no longer covers the branch", n, m, x0)
+        assert total[2] >= 1, ("the oracle did not reset its memory on this problem", n, m, x0, total)
         fs = [r["f"] for r in gpu[0]]
         assert all(b <= a for a, b in zip(fs, fs[1:])), (n, m, x0, fs)
         assert gpu[1].split(":")[0] == ref[1].split(":")[0], (n, m, x0, gpu[1], ref[1])

@@ -173,3 +173,33 @@ def test_errclb_messages(bad):
     s(n, m, x, l, u, nbd, f, g, factr, 1e-5, wa, iwa, task, -1, csave, lsave, isave, dsave)
     assert H.task_str(task) == want
     assert int(isave[41]) == k
+
+
+def test_event_counters_memory_reset_and_skipped_update():
+    """oracle_event_counts slots 2 (mainlb's "refresh the lbfgs memory" restarts) and 3 (skipped updates, :826-834)
+    fire on problems known to take those branches, and stay at zero on one that takes neither."""
+    from test_gpu_edge import _nonconvex
+    O.set_sum_mode(1)
+    try:
+        # REAL32 sample problem near convergence: lnsrlb meets an ascent direction with pairs in the memory
+        O.event_counts()
+        n, m = 1500, 5
+        x, l, u, nbd = H.rosenbrock_problem(n, dtype=np.float32)
+        H.run_driver(O.OracleSetulb(np.float32), O.rosenbrock_fg, n, m, x, l, u, nbd, 0.0, 0.0,
+                     stop=H.iteration_budget_stop(120), want_hash=False)
+        ev = O.event_counts()
+        assert ev[1] >= 1 and ev[2] >= ev[1], ev
+        # a concave share: s'y <= 0 along the step, the update is skipped
+        n, m = 400, 5
+        fg, mk = _nonconvex(n, 0, 0.5, 0.3)
+        x, l, u, nbd = mk()
+        tr = H.run_driver(O.OracleSetulb(), fg, n, m, x, l, u, nbd, 0.0, 0.0, stop=H.iteration_budget_stop(30),
+                          want_hash=False)
+        ev = O.event_counts()
+        assert ev[3] >= 1 and ev[3] == tr[0][-1]["nskip"], (ev, tr[0][-1])
+        # driver1: neither
+        x, l, u, nbd = H.rosenbrock_problem(25)
+        H.run_driver(O.OracleSetulb(), O.rosenbrock_fg, 25, 5, x, l, u, nbd, 1.0e7, 1.0e-5, want_hash=False)
+        assert O.event_counts()[2:4] == [0, 0]
+    finally:
+        O.set_sum_mode(0)
