@@ -105,17 +105,9 @@ static const char* fam_name[F_COUNT] = {
 
 // The scalar header of the state block straight into the host's pinned mirror, then a sequence word: the host waits
 // for that word instead of enqueueing a copy and synchronising the stream (a shorter round trip per setulb call).
+// The sequence number lives on the device, so that a captured CUDA graph publishes with the same fixed arguments.
 __global__ void __launch_bounds__(256) k_publish(const unsigned* src, unsigned* dst_host, int words, volatile unsigned long long* flag_host,
-                                                 unsigned long long seq) {
-    for (int q = threadIdx.x; q < words; q += blockDim.x) dst_host[q] = src[q];
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) *flag_host = seq;
-}
-
-// the same from inside a CUDA graph: the sequence number lives on the device (kernel arguments of a graph are fixed)
-__global__ void __launch_bounds__(256) k_publish_g(const unsigned* src, unsigned* dst_host, int words, volatile unsigned long long* flag_host,
-                                                   unsigned long long* counter) {
+                                                 unsigned long long* counter) {
     for (int q = threadIdx.x; q < words; q += blockDim.x) dst_host[q] = src[q];
     __threadfence_system();
     __syncthreads();
@@ -257,8 +249,6 @@ struct Engine : EngineBase {
         if (const char* e = getenv("LBFGSB_B200_NO_FUSION")) { if (e[0] == '1') fused = false; }
         fast = fused;   // the fast NEW_X pipeline is built from the fused passes
         if (const char* e = getenv("LBFGSB_B200_NO_FAST")) { if (e[0] == '1') fast = false; }
-        if (const char* e = getenv("LBFGSB_B200_NO_TIMERS")) { if (e[0] == '1') timers = false; }
-        if (const char* e = getenv("LBFGSB_B200_NO_SMALL_ROUNDS")) { if (e[0] == '1') { small_rounds = false; small_sort = false; } }
         if (const char* e = getenv("LBFGSB_B200_NO_BP_HINT")) { if (e[0] == '1') { bp_hint_ok = false; walk_gf_ok = false; } }
         if (!(mt == 5 ? set_smem_attrs<5>() : (mt == 10 ? set_smem_attrs<10>() : set_smem_attrs<20>()))) return false;
         for (int q = 0; q < F_COUNT; ++q) { fam_ms[q] = 0; fam_calls[q] = 0; }
@@ -273,8 +263,9 @@ struct Engine : EngineBase {
         if (!dalloc(&w.iwhere, (size_t)w.ldw * 4) || !dalloc(&w.state, (size_t)w.ldw)) return false;
         if (!dalloc(&w.part, sizeof(T) * LB_KMAX * LBFGSB_GRID) || !dalloc(&w.ipart, sizeof(i64) * LB_IMAX * LBFGSB_GRID)) return false;
         if (!dalloc(&w.part2, sizeof(T) * LB_KMAX * LBFGSB_GRID) || !dalloc(&w.ipart2, sizeof(i64) * LB_IMAX * LBFGSB_GRID)) return false;
-        if (!dalloc(&s_dev, sizeof(DevState<T>))) return false;
+        if (!dalloc(&s_dev, sizeof(DevState<T>)) || !dalloc(&pub_counter, 8) || !dalloc(&f_dev, sizeof(T))) return false;
         CK(cudaMemsetAsync(s_dev, 0, sizeof(DevState<T>), stream));
+        CK(cudaMemsetAsync(pub_counter, 0, 8, stream));
         {
             i64 lim = (i64)1 << 28;   // heap replay of tied breakpoints at the exit: up to 2.7e8 breakpoints by default
                                       // (on the device up to LB_TIE_DEVICE_MAX, beyond that on the engine's host thread)
@@ -288,7 +279,6 @@ struct Engine : EngineBase {
         CK(cudaHostAlloc((void**)&s_host, sizeof(DevState<T>) + 64, cudaHostAllocMapped));
         memset(s_host, 0, sizeof(DevState<T>) + 64);
         pub_flag = (volatile unsigned long long*)((char*)s_host + ((sizeof(DevState<T>) + 7) / 8) * 8);
-        if (const char* e = getenv("LBFGSB_B200_SYNC")) { if (e[0] == 'm') publish = false; }
         CK(cudaMallocHost((void**)&ctl_host, sizeof(SortCtl)));
         header_bytes = offsetof(DevState<T>, sy);
         // walk / compaction buffers
@@ -351,9 +341,7 @@ struct Engine : EngineBase {
     struct Mark { int ph; cudaEvent_t e; };
     std::vector<Mark> marks;
     double ph_time[3] = {0, 0, 0};
-    bool timers = true;
     void phase(int ph) {
-        if (!timers) return;
         Mark mk; mk.ph = ph; mk.e = get_event();
         cudaEventRecord(mk.e, stream);
         marks.push_back(mk);
@@ -400,28 +388,30 @@ struct Engine : EngineBase {
         }
         pending.clear();
     }
-    // state read-back: k_publish + a wait on the pinned sequence word; LBFGSB_B200_SYNC=memcpy: copy + stream synchronise
+    // state read-back: k_publish (enqueued here or captured in the iteration graph) + a wait on the pinned sequence word.
+    // Every k_publish that runs is waited for once, so the device counter and pub_expected advance together.
     volatile unsigned long long* pub_flag = nullptr;
-    unsigned long long pub_seq = 0;
-    bool publish = true;
-    bool sync_state(bool resolve = true) {
-        if (publish && pub_flag) {
-            pub_seq++;
-            k_publish<<<1, 256, 0, stream>>>((const unsigned*)s_dev, (unsigned*)s_host, (int)(header_bytes / 4), pub_flag, pub_seq);
-            launches++;
-            unsigned spins = 0;
-            while (*pub_flag != pub_seq) {
-                if ((++spins & 0x3fff) == 0) {   // a faulted kernel never publishes: ask the stream now and then
-                    cudaError_t q = cudaStreamQuery(stream);
-                    if (q != cudaSuccess && q != cudaErrorNotReady) { set_error("CUDA error %s while waiting for the state block", cudaGetErrorString(q)); return false; }
-                    if (q == cudaSuccess && *pub_flag != pub_seq) { set_error("the state block was not published (internal error)"); return false; }
-                }
+    unsigned long long* pub_counter = nullptr;
+    unsigned long long pub_expected = 0;
+    void enqueue_publish() {
+        k_publish<<<1, 256, 0, stream>>>((const unsigned*)s_dev, (unsigned*)s_host, (int)(header_bytes / 4), pub_flag, pub_counter);
+    }
+    bool wait_published() {
+        pub_expected++;
+        unsigned spins = 0;
+        while (*pub_flag != pub_expected) {
+            if ((++spins & 0x3fff) == 0) {   // a faulted kernel never publishes: ask the stream now and then
+                cudaError_t q = cudaStreamQuery(stream);
+                if (q != cudaSuccess && q != cudaErrorNotReady) { set_error("CUDA error %s while waiting for the state block", cudaGetErrorString(q)); return false; }
+                if (q == cudaSuccess && *pub_flag != pub_expected) { set_error("the state block was not published (internal error)"); return false; }
             }
-        } else {
-            CK(cudaMemcpyAsync(s_host, s_dev, header_bytes, cudaMemcpyDeviceToHost, stream));
-            CK(cudaStreamSynchronize(stream));
         }
         syncs++;
+        return true;
+    }
+    bool sync_state(bool resolve = true) {
+        enqueue_publish(); launches++;
+        if (!wait_published()) return false;
         if (profile && resolve) resolve_events();
         if (s_host->p2p_timeout) { set_error("a peer rank's reduction record did not arrive (sharded run over peer memory)"); return false; }
         return true;
@@ -778,7 +768,7 @@ struct Engine : EngineBase {
     }
     void enqueue_sort(typename Real<T>::key_t* k0, typename Real<T>::key_t* k1, int* v0, int* v1, SortCtl* ctl, i64 count) {
         typedef typename Real<T>::key_t K;
-        if (count <= LB_SMALL_SORT_MAX && small_sort) {   // (count = ctl->count: the callers pass what the device holds)
+        if (count <= LB_SMALL_SORT_MAX) {   // (count = ctl->count: the callers pass what the device holds)
             k_small_sort<K><<<1, 1024, 0, stream>>>(k0, k1, v0, v1, ctl); launches++;
             return;
         }
@@ -792,7 +782,6 @@ struct Engine : EngineBase {
         }
     }
     // a small round on a sharded problem (cauchy_walk_dist.cuh "Small rounds"): every rank scans the whole gathered list
-    bool small_rounds = true, small_sort = true;
     bool round_scan_gathered(i64 total) {
         typedef typename Real<T>::key_t K;
         const int col = s_host->col;
@@ -835,7 +824,7 @@ struct Engine : EngineBase {
     // one round on a sharded problem: this rank's breakpoints of the round are sorted in wb
     bool round_scan_sharded() {
         typedef typename Real<T>::key_t K;
-        if (small_rounds && s_host->walk_rcount > 0 && s_host->walk_rcount <= LB_RW_MAX) return round_scan_gathered(s_host->walk_rcount);
+        if (s_host->walk_rcount > 0 && s_host->walk_rcount <= LB_RW_MAX) return round_scan_gathered(s_host->walk_rcount);
         const int S = LB_DW_SAMPLES;
         // 2. splitters from regular samples
         begin(F_WALK_SCAN);
@@ -1055,23 +1044,35 @@ struct Engine : EngineBase {
             else if (ps == PAUSE_DELTA || ps == PAUSE_LSINIT) drop_events_from(ev_mid);
             resolve_events();
         }
+        return finish_call(false);
+    }
+    i64 fast_pauses = 0;
+
+    // The rest of a setulb call after its last read-back, from the state header in s_host: the general pipeline from
+    // where the fast one paused, the restored iterate, the body again after a restart, or lnsrlb's pending trial point.
+    // `stepped`: k_ls_step was already enqueued behind the read-back (the iteration graph) and took the step or unstep.
+    bool finish_call(bool stepped) {
         if (s_host->pause != PAUSE_NONE) {
             const int from = s_host->pause;
             fast_pauses++;
             s_resume<T><<<1, 32, 0, stream>>>(w); launches++;
             return enqueue_body(from);
         }
+        if (s_host->do_restore) {
+            begin(F_RESTORE); k_restore<T><<<LG>>>(w); end(F_RESTORE);
+            CK(cudaStreamSynchronize(stream));
+            if (profile) resolve_events();
+            x_changed = true; g_changed = true;
+        }
         if (s_host->restart) {
             // lnsrlb met an ascent direction at its first entry (:2247-2253) after the subspace pass had stepped
             // speculatively: x = t again before the iteration restarts (s_restart_body clears the flag)
-            if (s_host->do_unstep) { begin(F_LS_STEP); k_ls_step<T><<<LG>>>(w); end(F_LS_STEP); }
+            if (s_host->do_unstep && !stepped) { begin(F_LS_STEP); k_ls_step<T><<<LG>>>(w); end(F_LS_STEP); }
             begin(F_SCALAR); s_restart_body<T><<<1, 32, 0, stream>>>(w); end(F_SCALAR);
             return enqueue_body();
         }
-        return finish_step();
-    }
-    // lnsrlb's trial point after the state came back: nothing to do when the subspace pass already stepped
-    bool finish_step() {
+        if (stepped) return true;
+        // lnsrlb's trial point: nothing to do when the subspace pass already stepped
         if (s_host->do_unstep || (s_host->do_step && !s_host->step_done)) {
             begin(F_LS_STEP); k_ls_step<T><<<LG>>>(w); end(F_LS_STEP);
             CK(cudaStreamSynchronize(stream));
@@ -1080,29 +1081,20 @@ struct Engine : EngineBase {
         if (s_host->do_step) x_changed = true;
         return true;
     }
-    i64 fast_pauses = 0;
 
     // ---- device-resident iteration: the caller's loop as one CUDA graph per step (kernels_dense.cuh g_ls_trial / g_head) ----
     // Graph = [objective kernels -> g, f_dev] [k_ls_trial, g_ls_trial: FG_LNSRCH entry] [g_head .. f_tail: NEW_X entry, fast
-    // pipeline] [k_ls_step: the next trial point] [k_publish_g].  One launch and one read-back per step; whatever the fast
+    // pipeline] [k_ls_step: the next trial point] [k_publish].  One launch and one read-back per step; whatever the fast
     // pipeline does not cover (pause, restart, restore) is finished by the general pipeline on the host, as in call().
     cudaGraphExec_t iter_graph = nullptr;
-    unsigned long long* pub_count_dev = nullptr;
-    unsigned long long pub_count = 0;
-    T* f_dev = nullptr;
+    T* f_dev = nullptr;   // f of the objective callback of minimize_graph
     i64 graph_launches_per_step = 0, graph_steps = 0;
     template <typename FGE>
     bool build_iter_graph(FGE fg, void* user, int max_iter, int max_fg) {
         if (iter_graph) { cudaGraphExecDestroy(iter_graph); iter_graph = nullptr; }
-        if (!pub_count_dev) {
-            if (!dalloc(&pub_count_dev, 8) || !dalloc(&f_dev, sizeof(T))) return false;
-            CK(cudaMemsetAsync(pub_count_dev, 0, 8, stream));
-            pub_count = 0;
-        }
         w.bp_hint = 0;
         cudaGraph_t graph = nullptr;
         CK(cudaStreamBeginCapture(stream, cudaStreamCaptureModeRelaxed));
-        const i64 l0 = launches;
         int rc = fg(user, n, w.x, w.g, f_dev, (void*)stream);
         k_ls_trial<T><<<LG>>>(w);
         g_ls_trial<T><<<LS>>>(w, dist(), f_dev);
@@ -1114,8 +1106,7 @@ struct Engine : EngineBase {
         MTFUSED(launch_subsm_lsinit);
         f_tail<T><<<LS>>>(w, dist());
         k_ls_step<T><<<LG>>>(w);
-        k_publish_g<<<1, 256, 0, stream>>>((const unsigned*)s_dev, (unsigned*)s_host, (int)(header_bytes / 4), pub_flag + 1, pub_count_dev);
-        (void)l0;
+        enqueue_publish();
         graph_launches_per_step = 11;
         cudaError_t ce = cudaStreamEndCapture(stream, &graph);
         if (rc != 0 || ce != cudaSuccess || !graph) {
@@ -1133,41 +1124,12 @@ struct Engine : EngineBase {
     bool graph_step() {
         CK(cudaGraphLaunch(iter_graph, stream));
         launches += graph_launches_per_step; graph_steps++;
-        pub_count++;
-        volatile unsigned long long* fl = pub_flag + 1;
-        unsigned spins = 0;
-        while (*fl != pub_count) {
-            if ((++spins & 0x3fff) == 0) {
-                cudaError_t q = cudaStreamQuery(stream);
-                if (q != cudaSuccess && q != cudaErrorNotReady) { set_error("CUDA error %s in the iteration graph", cudaGetErrorString(q)); return false; }
-                if (q == cudaSuccess && *fl != pub_count) { set_error("the state block was not published by the iteration graph (internal error)"); return false; }
-            }
-        }
-        syncs++;
+        if (!wait_published()) return false;
         // what call() does after its read-back, for the call that ran last inside the graph
         for (auto& mk : marks) pool.push_back(mk.e);
         marks.clear();
         walked_now = false; body_ran = false;
-        if (s_host->gstage == 2) {
-            if (s_host->pause != PAUSE_NONE) {
-                const int from = s_host->pause;
-                fast_pauses++;
-                s_resume<T><<<1, 32, 0, stream>>>(w); launches++;
-                if (!enqueue_body(from)) return false;
-            } else if (s_host->restart) {
-                s_restart_body<T><<<1, 32, 0, stream>>>(w); launches++;
-                if (!enqueue_body()) return false;
-            }
-        } else {
-            if (s_host->do_restore) {
-                k_restore<T><<<LG>>>(w); launches++;
-                CK(cudaStreamSynchronize(stream));
-            }
-            if (s_host->restart) {
-                s_restart_body<T><<<1, 32, 0, stream>>>(w); launches++;
-                if (!enqueue_body()) return false;
-            }
-        }
+        if (!finish_call(true)) return false;
         resolve_phases();
         return check_launch();
     }
@@ -1235,18 +1197,7 @@ struct Engine : EngineBase {
             if (!site(site_lstrial())) return false;
             begin(F_SCALAR); s_ls_trial<T><<<LS>>>(w, dist(), 1, *f); end(F_SCALAR);
             phase(PH_END);
-            if (!sync_state()) return false;
-            if (s_host->do_restore) {
-                begin(F_RESTORE); k_restore<T><<<LG>>>(w); end(F_RESTORE);
-                CK(cudaStreamSynchronize(stream));
-                if (profile) resolve_events();
-                x_changed = true; g_changed = true;
-            }
-            if (!finish_step()) return false;
-            if (s_host->restart) {
-                begin(F_SCALAR); s_restart_body<T><<<1, 32, 0, stream>>>(w); end(F_SCALAR);
-                if (!enqueue_body()) return false;
-            }
+            if (!sync_state() || !finish_call(false)) return false;
         } else if (fast && s_host->cnstnd) {   // NEW_X, fast pipeline
             if (!fast_newx(*f)) return false;
         } else {   // NEW_X
@@ -1514,6 +1465,19 @@ static void setulb_dev_impl(lbfgsb_dev_t* hh, T* x, const T* l, const T* u, cons
 // The task loop of the reference's sample programs (test/driver1.f90:263-292, driver2.f90:112-190) as a
 // library call (the reference's own @todo, src/lbfgsb.f90:36-37).
 // ---------------------------------------------------------------------------
+// the caller's limits at NEW_X (driver2.f90:174-181): the STOP text to issue, or nullptr
+static const char* limit_stop(const int32_t* isave, int32_t max_iter, int32_t max_fg) {
+    const char* stop = nullptr;
+    if (max_fg > 0 && isave[33] >= max_fg) stop = "STOP: TOTAL NO. of f AND g EVALUATIONS EXCEEDS LIMIT";   // driver2.f90:176
+    if (max_iter > 0 && isave[29] >= max_iter) stop = "STOP: TOTAL NO. of ITERATIONS REACHED LIMIT";
+    return stop;
+}
+// return code of a finished loop: 0 converged, 1 abnormal line search, 2 error or STOP of a failed callback
+static int task_return_code(const char* task) {
+    if (pre60(task, "CONV")) return 0;
+    if (pre60(task, "ABNO")) return 1;
+    return 2;
+}
 template <typename T, typename FG>
 static int minimize_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, const int32_t* nbd, FG fg, void* user, T factr, T pgtol,
                          int32_t max_iter, int32_t max_fg, int32_t iprint, T* f, T* g, char* task, char* csave, int32_t* lsave,
@@ -1530,19 +1494,13 @@ static int minimize_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, const in
                 return 2;
             }
         } else if (pre60(task, "NEW_X")) {
-            const char* stop = nullptr;
-            if (max_fg > 0 && isave[33] >= max_fg) stop = "STOP: TOTAL NO. of f AND g EVALUATIONS EXCEEDS LIMIT";   // driver2.f90:176
-            if (max_iter > 0 && isave[29] >= max_iter) stop = "STOP: TOTAL NO. of ITERATIONS REACHED LIMIT";
-            if (stop) {
+            if (const char* stop = limit_stop(isave, max_iter, max_fg)) {
                 put60(task, stop);
                 setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
                 return 0;
             }
-        } else break;
+        } else return task_return_code(task);
     }
-    if (pre60(task, "CONV")) return 0;
-    if (pre60(task, "ABNO")) return 1;
-    return 2;
 }
 
 // The same loop kept on the device: the objective callback only ENQUEUES work on the given stream and leaves f in device
@@ -1556,18 +1514,10 @@ static int minimize_graph_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, co
     Engine<T>* e = (Engine<T>*)h;
     if (!e || e->real_kind != (int)sizeof(T) || !fg) { put60(task, "ERROR: INVALID LBFGSB_B200 HANDLE"); return 2; }
     const int32_t iprint = -1;
-    T* fd = nullptr;
     auto eval_host = [&]() -> bool {   // one evaluation outside the graph: f comes back to the host
-        if (!fd) { if (cudaMalloc((void**)&fd, sizeof(T)) != cudaSuccess) return false; }
-        if (fg(user, e->n, x, g, fd, (void*)e->stream) != 0) return false;
-        if (cudaMemcpyAsync(f, fd, sizeof(T), cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) return false;
+        if (fg(user, e->n, x, g, e->f_dev, (void*)e->stream) != 0) return false;
+        if (cudaMemcpyAsync(f, e->f_dev, sizeof(T), cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) return false;
         return cudaStreamSynchronize(e->stream) == cudaSuccess;
-    };
-    auto fail = [&]() {
-        put60(task, "STOP: THE OBJECTIVE CALLBACK FAILED");
-        setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
-        if (fd) cudaFree(fd);
-        return 2;
     };
     put60(task, "START");
     bool graph_ok = false, graph_tried = false;
@@ -1584,29 +1534,25 @@ static int minimize_graph_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, co
                 e->w.x = x; e->w.l = l; e->w.u = u; e->w.nbd = nbd; e->w.g = g; e->w.bp_hint = 0;
                 bool ok = true;
                 while (ok && e->s_host->task == TK_FG_LNSRCH) ok = e->graph_step();
-                if (!ok) { put60(task, "ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)"); if (fd) cudaFree(fd); return 2; }
+                if (!ok) { put60(task, "ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)"); return 2; }
                 *f = e->s_host->f;
                 export_state<T>(e, task, csave, lsave, isave, dsave);
             }
         }
         if (pre60(task, "FG")) {
-            if (!eval_host()) return fail();
+            if (!eval_host()) {
+                put60(task, "STOP: THE OBJECTIVE CALLBACK FAILED");
+                setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
+                return 2;
+            }
         } else if (pre60(task, "NEW_X")) {
-            const char* stop = nullptr;
-            if (max_fg > 0 && isave[33] >= max_fg) stop = "STOP: TOTAL NO. of f AND g EVALUATIONS EXCEEDS LIMIT";   // driver2.f90:176
-            if (max_iter > 0 && isave[29] >= max_iter) stop = "STOP: TOTAL NO. of ITERATIONS REACHED LIMIT";
-            if (stop) {
+            if (const char* stop = limit_stop(isave, max_iter, max_fg)) {
                 put60(task, stop);
                 setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
-                if (fd) cudaFree(fd);
                 return 0;
             }
-        } else break;
+        } else return task_return_code(task);
     }
-    if (fd) cudaFree(fd);
-    if (pre60(task, "CONV")) return 0;
-    if (pre60(task, "ABNO")) return 1;
-    return 2;
 }
 
 // ---------------------------------------------------------------------------
