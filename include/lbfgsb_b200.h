@@ -239,7 +239,10 @@ int lbfgsb_problem_quadratic_f32(int64_t n, const float* x_dev, float* g_dev, fl
  * terminal one ('CONVERGENCE...', 'ABNORMAL...', 'ERROR...', 'STOP...') are left alone, so the caller simply keeps
  * calling until lbfgsb_batch_counts reports no 'FG' and no 'NEW_X' task.  'STOP' with task(7:9)='CPU' restores the
  * previous iterate of that problem (:565-571).  Equal breakpoints are taken in hpsolb's order (the Cauchy search of
- * a small problem is the reference's own sequential loop, :1378-1497). */
+ * a small problem is the reference's own sequential loop, :1378-1497).
+ * A call works on the batch's stream (lbfgsb_batch_stream) and reads f_dev and g_dev there: the caller must order
+ * that stream after the writes of f and g (an event recorded after the objective and waited on by the batch's
+ * stream, or the objective enqueued on that stream itself).  The call synchronises the stream before it returns. */
 typedef struct lbfgsb_batch lbfgsb_batch_t;
 lbfgsb_batch_t* lbfgsb_batch_create(int32_t nprob, int64_t n, int32_t m, int32_t real_kind, void* cuda_stream);
 void lbfgsb_batch_destroy(lbfgsb_batch_t* h);
@@ -257,6 +260,11 @@ void* lbfgsb_batch_fg_mask(lbfgsb_batch_t* h);
 /* iwhere of every problem copied to the host, int32 [nprob][n] -- what the reference keeps in iwa(2n+1:3n)
  * (src/lbfgsb.f90:258; codes -3, -1, 0, 1, 2, 3 of cauchy :1203-1213).  Returns 0 on success. */
 int lbfgsb_batch_get_iwhere(lbfgsb_batch_t* h, int32_t* iwhere_host);
+/* diagnostics: copy `bytes` of one problem's work vector to dst_dev (device), with the `which` codes of
+ * lbfgsb_dev_vector_copy (0 z, 1 r, 2 d, 3 t, 4 xp, 7 iwhere, 8 the previous gradient: ldw = roundup(n, 32) elements;
+ * 5 ws, 6 wy: m columns of ldw reals, column j of the S/Y ring at j * ldw).  Returns nonzero for a problem out of
+ * range, an unknown code or a byte count beyond that problem's slice. */
+int lbfgsb_batch_vector_copy(lbfgsb_batch_t* h, int32_t problem, int32_t which, void* dst_dev, int64_t bytes);
 /* the sample objective (test/driver1.f90:274-289) for a batch: problem p from x_dev[p][.] into g_dev[p][.], f_dev[p];
  * mask_dev (may be NULL): int32 [nprob], problems with 0 are skipped */
 int lbfgsb_problem_rosenbrock_batch_f64(int32_t nprob, int64_t n, const double* x_dev, double* g_dev, double* f_dev,

@@ -125,6 +125,7 @@ def lib():
         L.lbfgsb_batch_get_iwhere.argtypes = [C.c_void_p, C.c_void_p]
         L.lbfgsb_batch_fg_mask.restype = C.c_void_p
         L.lbfgsb_batch_fg_mask.argtypes = [C.c_void_p]
+        L.lbfgsb_batch_vector_copy.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64]
         for sfx in ("f64", "f32"):
             getattr(L, "lbfgsb_batch_setulb_dev_" + sfx).restype = None
             getattr(L, "lbfgsb_batch_setulb_dev_" + sfx).argtypes = [C.c_void_p] * 14
@@ -520,6 +521,14 @@ class BatchProblem:
         self._fg = getattr(lib(), "lbfgsb_problem_rosenbrock_batch_" + sfx)
         self.stream = lib().lbfgsb_batch_stream(C.c_void_p(self.h))
         self.fg_mask_ptr = lib().lbfgsb_batch_fg_mask(C.c_void_p(self.h))
+        self._ext = None      # torch's view of the batch's stream, made at the first call
+
+    def _after_torch(self):
+        """Orders the batch's stream after the work enqueued so far on torch's current stream."""
+        import torch
+        if self._ext is None:
+            self._ext = torch.cuda.ExternalStream(self.stream)
+        self._ext.wait_stream(torch.cuda.current_stream())
 
     def task_str(self, p):
         return bytes(self.task[p]).decode().rstrip()
@@ -530,6 +539,9 @@ class BatchProblem:
         self.task[p, :len(b)] = np.frombuffer(b, dtype=np.uint8)
 
     def setulb_dev(self, x, l, u, nbd, f, g, factr, pgtol):
+        """One call for the whole batch.  The batch's stream first waits for torch's current stream, so f and g written
+        there by a torch objective are complete before the kernel reads them."""
+        self._after_torch()
         fa, pg = self._cr(factr), self._cr(pgtol)
         self._fn(C.c_void_p(self.h), C.c_void_p(x.data_ptr()), C.c_void_p(l.data_ptr()), C.c_void_p(u.data_ptr()),
                  C.c_void_p(nbd.data_ptr()), C.c_void_p(f.data_ptr()), C.c_void_p(g.data_ptr()), C.byref(fa), C.byref(pg),
@@ -543,6 +555,20 @@ class BatchProblem:
         out = np.empty((self.nprob, self.n), dtype=np.int32)
         if lib().lbfgsb_batch_get_iwhere(C.c_void_p(self.h), _p(out)) != 0:
             raise LbfgsbB200Error("lbfgsb_batch_get_iwhere failed")
+        return out
+
+    def vector(self, p, which, count=None):
+        """Copy of problem p's slice of a work vector (diagnostics; codes of DeviceProblem.vector): n elements by
+        default; ws (5) and wy (6) hold m columns of ldw = roundup(n, 32) reals, so pass count = m * ldw for them.
+        A problem out of range or a count beyond the problem's slice raises."""
+        import torch
+        k = self.n if count is None else int(count)
+        tdt = torch.int32 if which == 7 else {np.dtype(np.float64): torch.float64, np.dtype(np.float32): torch.float32}[self.dtype]
+        out = torch.empty(k, dtype=tdt, device="cuda")
+        self._after_torch()     # the copy runs on the batch's stream
+        if lib().lbfgsb_batch_vector_copy(C.c_void_p(self.h), int(p), int(which), C.c_void_p(out.data_ptr()),
+                                          C.c_int64(out.numel() * out.element_size())) != 0:
+            raise LbfgsbB200Error("lbfgsb_batch_vector_copy failed: " + last_error())
         return out
 
     def counts(self):

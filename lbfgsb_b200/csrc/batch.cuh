@@ -655,6 +655,15 @@ template <typename T> __device__ void stage3_out(DevState<T>* s, BatchSm<T>& sm)
     __syncthreads();
 }
 
+// The restart flag, as every thread of the CTA saw it after the step.  Thread 0 clears s->restart next (begin_body):
+// each thread takes the flag into a register and the barrier keeps that store behind every thread's read, so no
+// warp can see the cleared flag and leave while the others run the restarted iteration without it.
+template <typename T> __device__ __forceinline__ bool restart_taken(const DevState<T>* s) {
+    const int rs = s->restart;
+    __syncthreads();
+    return rs != 0;
+}
+
 // ---- prelims + first lnsrlb (:601-773): the general pipeline of Engine::enqueue_body inside one CTA --------------
 template <typename T, int MT>
 __device__ void body(Wk<T>& w, T* bpt, int* bpo, T* delta, BatchSm<T>& sm) {
@@ -713,7 +722,7 @@ __device__ void body(Wk<T>& w, T* bpt, int* bpo, T* delta, BatchSm<T>& sm) {
             __syncthreads();
         }
         ls_step<T>(w);
-        if (!s->restart) return;
+        if (!restart_taken(s)) return;
         if (threadIdx.x == 0) { s->go = 1; s->pause = 0; s->classify_done = 0; begin_body<T>(s); }   // s_restart_body
     }
 }
@@ -774,7 +783,7 @@ __global__ void __launch_bounds__(LBFGSB_BLOCK) k_batch_setulb(BatchWk<T> bw) {
         __syncthreads();
         if (s->do_restore) batch::restore<T>(w);
         batch::ls_step<T>(w);
-        if (s->restart) {
+        if (batch::restart_taken(s)) {
             if (threadIdx.x == 0) { s->go = 1; s->pause = 0; s->classify_done = 0; begin_body<T>(s); }
             batch::body<T, MT>(w, bpt, bpo, delta, sm);
         }

@@ -2097,6 +2097,28 @@ struct BatchEngine : BatchBase {
         }
         return true;
     }
+    // one problem's slice of a work vector (lbfgsb_batch_vector_copy), copied on the batch's stream
+    int vector_copy(int p, int which, void* dst, i64 bytes) {
+        if (p < 0 || p >= bw.nprob) { set_error("lbfgsb_batch_vector_copy: problem %d out of range [0, %d)", p, bw.nprob); return 1; }
+        const i64 o = (i64)p * bw.ldw, vb = bw.ldw * (i64)sizeof(T);
+        const void* src = nullptr;
+        i64 cap = vb;
+        switch (which) {
+            case 0: src = bw.z + o; break;
+            case 1: src = bw.r + o; break;
+            case 2: src = bw.d + o; break;
+            case 3: src = bw.t + o; break;
+            case 4: src = bw.xp + o; break;
+            case 5: src = bw.ws + o * bw.m; cap = bw.m * vb; break;
+            case 6: src = bw.wy + o * bw.m; cap = bw.m * vb; break;
+            case 7: src = bw.iwhere + o; cap = bw.ldw * 4; break;
+            case 8: src = bw.gold + o; break;
+            default: set_error("lbfgsb_batch_vector_copy: no vector %d", which); return 1;
+        }
+        if (bytes > cap) { set_error("lbfgsb_batch_vector_copy: %lld bytes requested, vector %d of a problem holds %lld", (long long)bytes, which, (long long)cap); return 1; }
+        if (cudaMemcpyAsync(dst, src, (size_t)bytes, cudaMemcpyDeviceToDevice, stream) != cudaSuccess) return 1;
+        return cudaStreamSynchronize(stream) != cudaSuccess;
+    }
 };
 
 // sample objective for a batch (test/driver1.f90:274-289, one CTA per problem): the arithmetic and the summation shape
@@ -2651,6 +2673,12 @@ int lbfgsb_batch_get_iwhere(lbfgsb_batch_t* h, int32_t* iwhere_host) {
     else { BatchEngine<float>* e = (BatchEngine<float>*)b; src = e->bw.iwhere; ldw = e->bw.ldw; n = e->bw.n; nprob = e->bw.nprob; st = e->stream; }
     if (cudaMemcpy2DAsync(iwhere_host, (size_t)n * 4, src, (size_t)ldw * 4, (size_t)n * 4, (size_t)nprob, cudaMemcpyDeviceToHost, st) != cudaSuccess) return 1;
     return cudaStreamSynchronize(st) != cudaSuccess;
+}
+int lbfgsb_batch_vector_copy(lbfgsb_batch_t* h, int32_t problem, int32_t which, void* dst_dev, int64_t bytes) {
+    BatchBase* b = (BatchBase*)h;
+    if (!b || !dst_dev || bytes < 0) return 1;
+    if (b->real_kind == 8) return ((BatchEngine<double>*)b)->vector_copy(problem, which, dst_dev, bytes);
+    return ((BatchEngine<float>*)b)->vector_copy(problem, which, dst_dev, bytes);
 }
 void* lbfgsb_batch_stream(lbfgsb_batch_t* h) {
     BatchBase* b = (BatchBase*)h;

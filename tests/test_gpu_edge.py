@@ -107,10 +107,12 @@ def test_nonconvex_objective_with_skips_and_line_search_backtracks(n, m, seed, s
     assert any(r["iback"] > 0 for r in ref[0][:14])
 
 
-def sweep_problem(seed):
-    """(n, m, fg, mk) of a seeded mixed-bound problem: nbd in {0, 1, 2, 3}, 3 % fixed variables, a coupled quartic."""
+def sweep_problem(seed, n=None):
+    """(n, m, fg, mk) of a seeded mixed-bound problem: nbd in {0, 1, 2, 3}, 3 % fixed variables, a coupled quartic.
+    n: the seed's own size in [60, 6000) unless given."""
     rng = np.random.default_rng(seed)
-    n = int(rng.integers(60, 6000))
+    n_seed = int(rng.integers(60, 6000))
+    n = n_seed if n is None else int(n)
     m = int(rng.integers(1, 13))
     a = rng.uniform(0.5, 3.0, n)
     b = rng.uniform(-2.0, 2.0, n)
