@@ -32,7 +32,7 @@ module lbfgsb_module
    public :: setulb, setulb_dev
    public :: lbfgsb_dev_create, lbfgsb_dev_destroy, lbfgsb_host_release
    public :: lbfgsb_dev_set_tie_limit, lbfgsb_dev_checkpoint_write, lbfgsb_dev_checkpoint_read
-   public :: lbfgsb_minimize_graph_dev
+   public :: lbfgsb_minimize_graph_dev, lbfgsb_batch_minimize_graph_dev
    public :: lbfgsb_batch_create, lbfgsb_batch_destroy, setulb_batch_dev, lbfgsb_batch_counts, lbfgsb_batch_get_iwhere
 
    interface
@@ -131,6 +131,28 @@ module lbfgsb_module
          integer(c_int32_t), intent(inout) :: lsave(4), isave(44)
          integer(c_int) :: rc
       end function lbfgsb_minimize_graph_dev
+
+      !> The whole task loop of a batch on the device (CUDA-graph launches of up to 128 calls each); every problem starts
+      !> from 'START'.  fg is a C function pointer int fg(void* user, int32_t nprob, int64_t n, const real* x_dev,
+      !> real* g_dev, real* f_dev, const int32_t* mask_dev, void* cuda_stream) that only enqueues kernels for the problems
+      !> with mask_dev(p) = 1 (c_funloc of a bind(C) procedure).  Arrays as for setulb_batch_dev; f is a device pointer.
+#ifdef REAL32
+      function lbfgsb_batch_minimize_graph_dev(h, x, l, u, nbd, f, g, fg, user, factr, pgtol, max_iter, max_fg, task, &
+         csave, lsave, isave, dsave) result(rc) bind(C, name='lbfgsb_batch_minimize_graph_f32')
+#else
+      function lbfgsb_batch_minimize_graph_dev(h, x, l, u, nbd, f, g, fg, user, factr, pgtol, max_iter, max_fg, task, &
+         csave, lsave, isave, dsave) result(rc) bind(C, name='lbfgsb_batch_minimize_graph_f64')
+#endif
+         import :: c_int32_t, c_char, c_ptr, c_funptr, c_int, wp
+         type(c_ptr), value :: h, x, l, u, nbd, f, g, user
+         type(c_funptr), value :: fg
+         real(wp), value :: factr, pgtol
+         integer(c_int32_t), value :: max_iter, max_fg
+         character(kind=c_char), intent(inout) :: task(60, *), csave(60, *)
+         integer(c_int32_t), intent(inout) :: lsave(4, *), isave(44, *)
+         real(wp), intent(inout) :: dsave(29, *)
+         integer(c_int) :: rc
+      end function lbfgsb_batch_minimize_graph_dev
 
       !> Batched small problems: nprob independent problems of the same n and m, one call advances every problem from
       !> its own task to its next return point (the caller's loop of test/driver1.f90:263-292, many times over).

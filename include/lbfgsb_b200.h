@@ -271,6 +271,44 @@ int lbfgsb_problem_rosenbrock_batch_f64(int32_t nprob, int64_t n, const double* 
                                         const int32_t* mask_dev, void* cuda_stream);
 int lbfgsb_problem_rosenbrock_batch_f32(int32_t nprob, int64_t n, const float* x_dev, float* g_dev, float* f_dev,
                                         const int32_t* mask_dev, void* cuda_stream);
+/* The whole task loop of a batch on the device.  Every problem starts from 'START' (through lbfgsb_batch_setulb_dev_*,
+ * so errclb's errors land in task, isave(35) and isave(42) as there); then, while a problem is at 'FG' or 'NEW_X', one
+ * graph launch runs up to 128 calls of the loop [fg] [setulb call of every problem] on the device, and the host reads one
+ * small result per launch; at the end the state of every problem is exported once.  The results are bit for bit those of
+ * the same loop run call by call on the host (Python BatchProblem.solve) with the same objective and limits.
+ * Limits, per problem, at 'NEW_X' (as lbfgsb_minimize_dev_*): iter >= max_iter gives 'STOP: TOTAL NO. of ITERATIONS
+ * REACHED LIMIT', otherwise nfgv >= max_fg 'STOP: TOTAL NO. of f AND g EVALUATIONS EXCEEDS LIMIT'; a limit <= 0 is no limit.
+ * A stopped problem's state is left as that 'NEW_X' left it, and a later lbfgsb_batch_setulb_dev_* call treats it as
+ * ended by the caller's STOP.
+ * The objective contract:
+ *   - fg only ENQUEUES work on cuda_stream (the batch's stream) and is captured into a CUDA graph: it must not allocate,
+ *     synchronise or read anything back.  It is called once per graph build, not once per call.
+ *   - It must evaluate f_dev[p] and g_dev[p][.] at x_dev[p][.] for every problem p with mask_dev[p] == 1 (mask_dev is
+ *     lbfgsb_batch_fg_mask).  For every other problem it must leave f and g untouched or recompute them at the same x.
+ *     lbfgsb_problem_rosenbrock_batch_* meets this contract.
+ *   - It returns 0; anything else aborts the solve.
+ * The graph is kept on the handle and rebuilt only when x, l, u, nbd, f, g, fg, user, factr, pgtol or a limit changes.
+ * As for lbfgsb_batch_setulb_dev_*, the caller orders the batch's stream after its writes of x, l, u and nbd.
+ * Conditional graph nodes need a CUDA 12.3 or later driver; an older one gives 2.
+ * Returns 0 when the loop ran (each task then holds the problem's end: CONVERGENCE, ABNORMAL, ERROR or a limit's STOP);
+ * 2 when the objective failed or could not be captured ('STOP: THE OBJECTIVE CALLBACK FAILED' in every task that had not
+ * finished) or on a CUDA failure ('ERROR: CUDA FAILURE ...'), with the reason in lbfgsb_b200_last_error.  An invalid
+ * handle, or one of the other real kind, gives 2 and 'ERROR: INVALID LBFGSB_B200 HANDLE' in every task. */
+typedef int (*lbfgsb_batch_fg_enqueue_f64)(void* user, int32_t nprob, int64_t n, const double* x_dev, double* g_dev,
+                                           double* f_dev, const int32_t* mask_dev, void* cuda_stream);
+typedef int (*lbfgsb_batch_fg_enqueue_f32)(void* user, int32_t nprob, int64_t n, const float* x_dev, float* g_dev,
+                                           float* f_dev, const int32_t* mask_dev, void* cuda_stream);
+int lbfgsb_batch_minimize_graph_f64(lbfgsb_batch_t* h, double* x_dev, const double* l_dev, const double* u_dev,
+                                    const int32_t* nbd_dev, double* f_dev, double* g_dev, lbfgsb_batch_fg_enqueue_f64 fg,
+                                    void* user, double factr, double pgtol, int32_t max_iter, int32_t max_fg, char* task,
+                                    char* csave, int32_t* lsave, int32_t* isave, double* dsave);
+int lbfgsb_batch_minimize_graph_f32(lbfgsb_batch_t* h, float* x_dev, const float* l_dev, const float* u_dev,
+                                    const int32_t* nbd_dev, float* f_dev, float* g_dev, lbfgsb_batch_fg_enqueue_f32 fg,
+                                    void* user, float factr, float pgtol, int32_t max_iter, int32_t max_fg, char* task,
+                                    char* csave, int32_t* lsave, int32_t* isave, float* dsave);
+/* counters since the batch was created: graphs built, graph launches, and setulb calls made by
+ * lbfgsb_batch_minimize_graph_* (START included) */
+int lbfgsb_batch_graph_stats(lbfgsb_batch_t* h, int64_t* graph_builds, int64_t* graph_launches, int64_t* calls);
 
 /* ---- single-kernel entry points for the per-routine parity tests (device pointers) ---------- */
 int lbfgsb_test_projgr_f64(int64_t n, const double* l, const double* u, const int32_t* nbd, const double* x,

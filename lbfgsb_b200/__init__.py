@@ -126,6 +126,7 @@ def lib():
         L.lbfgsb_batch_fg_mask.restype = C.c_void_p
         L.lbfgsb_batch_fg_mask.argtypes = [C.c_void_p]
         L.lbfgsb_batch_vector_copy.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64]
+        L.lbfgsb_batch_graph_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         for sfx in ("f64", "f32"):
             getattr(L, "lbfgsb_batch_setulb_dev_" + sfx).restype = None
             getattr(L, "lbfgsb_batch_setulb_dev_" + sfx).argtypes = [C.c_void_p] * 14
@@ -603,6 +604,57 @@ class BatchProblem:
                 if max_iter > 0:
                     for p in np.nonzero((self.task[:, 0] == 78) & (self.isave[:, 29] >= max_iter))[0]:
                         self.set_task(int(p), "STOP: TOTAL NO. of ITERATIONS REACHED LIMIT")
+
+    def rosenbrock_enqueue(self):
+        """The sample objective as an objective for solve_graph: the batched Rosenbrock kernel, masked by the mask it is
+        given (the batch's fg_mask), enqueued on the stream it is given.  The same function object on every call, so a
+        solve_graph with the default objective reuses its graph."""
+        if getattr(self, "_rosen_enq", None) is None:
+            fn, nprob, n = self._fg, self.nprob, self.n
+
+            def enq(xp, gp, fp, mp, stream):
+                if fn(nprob, n, C.c_void_p(xp), C.c_void_p(gp), C.c_void_p(fp), C.c_void_p(mp), C.c_void_p(stream)) != 0:
+                    raise LbfgsbB200Error("batched objective kernel failed")
+            self._rosen_enq = enq
+        return self._rosen_enq
+
+    def solve_graph(self, x, l, u, nbd, f, g, factr, pgtol, fg_enqueue=None, max_iter=0, max_fg=0):
+        """lbfgsb_batch_minimize_graph_*: the task loop of solve run on the device, as CUDA-graph launches of up to 128
+        calls each.  Every problem starts from 'START'.  fg_enqueue(x_ptr, g_ptr, f_ptr, mask_ptr, stream) only enqueues
+        the objective's kernels on `stream` for the problems whose mask entry is 1; it is captured once per graph build
+        (include/lbfgsb_b200.h section 6).  Default: the sample objective.  Limits as in lbfgsb_minimize_dev_* (max_iter
+        before max_fg at NEW_X; <= 0: none).  Returns the number of calls, like solve; raises when the C call returns
+        nonzero (a failed objective leaves 'STOP: THE OBJECTIVE CALLBACK FAILED' in the unfinished tasks)."""
+        fg_enqueue = fg_enqueue or self.rosenbrock_enqueue()
+        sfx, cr = _REAL[self.dtype]
+        CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p)
+        if getattr(self, "_graph_cb", (None, None))[0] is not fg_enqueue:
+            def _cb(user, nprob, n, xp, gp, fp, mp, stream):
+                try:
+                    fg_enqueue(xp, gp, fp, mp, stream)
+                    return 0
+                except Exception:  # noqa: BLE001
+                    return 1
+            # one C function pointer per objective: it is part of the key of the graph kept on the handle
+            self._graph_cb = (fg_enqueue, CB(_cb))
+        fn = getattr(lib(), "lbfgsb_batch_minimize_graph_" + sfx)
+        fn.restype = C.c_int
+        fn.argtypes = [C.c_void_p] * 7 + [CB, C.c_void_p, cr, cr, C.c_int32, C.c_int32] + [C.c_void_p] * 5
+        calls0 = self.graph_stats()[2]
+        self._after_torch()
+        rc = fn(C.c_void_p(self.h), C.c_void_p(x.data_ptr()), C.c_void_p(l.data_ptr()), C.c_void_p(u.data_ptr()),
+                C.c_void_p(nbd.data_ptr()), C.c_void_p(f.data_ptr()), C.c_void_p(g.data_ptr()), self._graph_cb[1], None,
+                cr(factr), cr(pgtol), int(max_iter), int(max_fg), _p(self.task), _p(self.csave), _p(self.lsave),
+                _p(self.isave), _p(self.dsave))
+        if rc != 0:
+            raise LbfgsbB200Error("lbfgsb_batch_minimize_graph_%s returned %d: %s" % (sfx, rc, last_error()))
+        return self.graph_stats()[2] - calls0
+
+    def graph_stats(self):
+        """(graphs built, graph launches, calls made by solve_graph) since the batch was created."""
+        a, b, c = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        lib().lbfgsb_batch_graph_stats(C.c_void_p(self.h), C.byref(a), C.byref(b), C.byref(c))
+        return a.value, b.value, c.value
 
     def close(self):
         if self.h:

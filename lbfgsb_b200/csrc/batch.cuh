@@ -36,8 +36,13 @@ struct BatchWk {
     const int* entry;                     // [nprob] what the caller's task asks for (BE_*)
     int* fgmask;                          // [nprob] out: 1 where the problem's new task asks for f and g
     T factr, pgtol;
+    // the task loop on the device (k_batch_setulb<T, MT, true>): entries come from each problem's own state block
+    int* stop;                            // [nprob] out: BS_* limit that stopped the problem at NEW_X, 0 while none did
+    int* loop;                            // [3] problems that returned with an FG or NEW_X task; calls and that count (k_batch_loop_*)
+    int max_iter, max_fg;                 // limits of limit_stop (engine.cu); <= 0: no limit
 };
 enum { BE_START = 0, BE_FG_START = 1, BE_FG_LNSRCH = 2, BE_NEW_X = 3, BE_STOP = 4, BE_STOP_CPU = 5, BE_OTHER = 6, BE_IDLE = 7 };
+enum { BS_NONE = 0, BS_ITER = 1, BS_FG = 2 };
 
 // shared scratch of one CTA (dynamic shared memory)
 template <typename T>
@@ -727,16 +732,40 @@ __device__ void body(Wk<T>& w, T* bpt, int* bpo, T* delta, BatchSm<T>& sm) {
     }
 }
 
+// The entry of a device-resident call, from the problem's own task as the previous call left it in the state block:
+// FG_START, FG_LNSRCH and NEW_X continue, everything else is finished.  At NEW_X the caller's limits apply as in
+// limit_stop (engine.cu): max_iter before max_fg; a stopped problem is recorded in bw.stop and its state block is left
+// as that NEW_X left it.  Every thread reads the state before the barrier, so no thread sees what thread 0 writes next.
+template <typename T>
+__device__ __forceinline__ int device_entry(const BatchWk<T>& bw, int p) {
+    const DevState<T>* s = bw.s + p;
+    const int task = s->task;
+    int e = BE_IDLE, stop = BS_NONE;
+    if (task == TK_FG_START) e = BE_FG_START;
+    else if (task == TK_FG_LNSRCH) e = BE_FG_LNSRCH;
+    else if (task == TK_NEW_X) {
+        if (bw.max_fg > 0 && s->nfgv >= bw.max_fg) stop = BS_FG;
+        if (bw.max_iter > 0 && s->iter >= bw.max_iter) stop = BS_ITER;
+        e = stop ? BE_IDLE : BE_NEW_X;
+    }
+    __syncthreads();
+    if (stop && threadIdx.x == 0) bw.stop[p] = stop;
+    return e;
+}
+
 }  // namespace batch
 
-// One reverse-communication call for the whole batch.
-template <typename T, int MT>
+// One reverse-communication call for the whole batch.  DEV: the entries come from the state blocks (batch::device_entry)
+// instead of the host's entry[], and every problem that returns with an FG or NEW_X task is counted in bw.loop[0].
+template <typename T, int MT, bool DEV = false>
 __global__ void __launch_bounds__(LBFGSB_BLOCK) k_batch_setulb(BatchWk<T> bw) {
     extern __shared__ __align__(16) unsigned char bsm_raw[];
     BatchSm<T>& sm = *reinterpret_cast<BatchSm<T>*>(bsm_raw);
     const int p = blockIdx.x;
     if (p >= bw.nprob) return;
-    const int entry = bw.entry[p];
+    int entry;
+    if constexpr (DEV) entry = batch::device_entry<T>(bw, p);
+    else entry = bw.entry[p];
     if (entry == BE_IDLE) { if (threadIdx.x == 0) bw.fgmask[p] = 0; return; }
     Wk<T> w;
     w.n = bw.n; w.ldw = bw.ldw; w.off = 0; w.m = bw.m;
@@ -804,4 +833,21 @@ __global__ void __launch_bounds__(LBFGSB_BLOCK) k_batch_setulb(BatchWk<T> bw) {
     }
     __syncthreads();
     if (threadIdx.x == 0) { bw.f[p] = s->f; bw.fgmask[p] = (s->task == TK_FG_START || s->task == TK_FG_LNSRCH) ? 1 : 0; }
+    if constexpr (DEV) {
+        if (threadIdx.x == 0 && (s->task == TK_FG_START || s->task == TK_FG_LNSRCH || s->task == TK_NEW_X)) atomicAdd(bw.loop, 1);
+    }
+}
+
+// The loop of lbfgsb_batch_minimize_graph_*: a graph launch runs [k_batch_loop_reset] then a WHILE node whose body is
+// [objective] [k_batch_setulb<T, MT, true>] [k_batch_loop_cond].  loop[0] counts the problems still at FG or NEW_X after
+// the call, loop[1] the calls of this launch, loop[2] keeps the last count for the host.  The body repeats while a
+// problem is active and the launch has made fewer than `cap` calls, so no launch runs unbounded.
+__global__ void k_batch_loop_reset(int* loop) { loop[1] = 0; }
+__global__ void k_batch_loop_cond(cudaGraphConditionalHandle h, int* loop, int cap) {
+    const int active = loop[0];
+    loop[0] = 0;
+    loop[2] = active;
+    const int calls = loop[1] + 1;
+    loop[1] = calls;
+    cudaGraphSetConditional(h, (active > 0 && calls < cap) ? 1u : 0u);
 }

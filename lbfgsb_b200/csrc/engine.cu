@@ -2040,9 +2040,11 @@ struct BatchEngine : BatchBase {
         return true;
     }
     ~BatchEngine() {
+        if (loop_exec) cudaGraphExecDestroy(loop_exec);
         for (void* p : allocs) cudaFree(p);
         if (hdr_host) cudaFreeHost(hdr_host);
         if (entry_host) cudaFreeHost(entry_host);
+        if (loop_host) cudaFreeHost(loop_host);
         if (own_stream && stream) cudaStreamDestroy(stream);
     }
     bool call(T* x, const T* l, const T* u, const int32_t* nbd, T* f, T* g, T factr, T pgtol, char* task, char* csave, int32_t* lsave,
@@ -2119,6 +2121,164 @@ struct BatchEngine : BatchBase {
         if (cudaMemcpyAsync(dst, src, (size_t)bytes, cudaMemcpyDeviceToDevice, stream) != cudaSuccess) return 1;
         return cudaStreamSynchronize(stream) != cudaSuccess;
     }
+
+    // ---- the task loop on the device (lbfgsb_batch_minimize_graph_*) ----
+    // One graph = [k_batch_loop_reset] -> WHILE { [objective, mask = fgmask] [k_batch_setulb<T, MT, true>] [k_batch_loop_cond] },
+    // instantiated once and kept while the captured arguments stay the same.
+    static constexpr int kLoopCallCap = 128;   // calls per graph launch at most
+    struct LoopKey {
+        T* x; const T *l, *u; const int32_t* nbd; T *f, *g;
+        void *fg, *user;
+        T factr, pgtol;
+        int32_t max_iter, max_fg;
+    };
+    cudaGraphExec_t loop_exec = nullptr;
+    LoopKey loop_key;
+    int* loop_host = nullptr;                  // pinned [4 + nprob]: loop[0..2] of the device, then the BS_* codes
+    i64 graph_builds = 0, graph_launches = 0, graph_calls = 0;
+
+    template <int MT> void launch_dev_entry() {
+        k_batch_setulb<T, MT, true><<<bw.nprob, LBFGSB_BLOCK, sizeof(BatchSm<T>), stream>>>(bw);
+    }
+    // 0 built; 1 the objective failed or could not be captured; 2 CUDA failure
+    template <typename FGE>
+    int build_loop_graph(FGE fg, void* user) {
+        if (loop_exec) { cudaGraphExecDestroy(loop_exec); loop_exec = nullptr; }
+        cudaGraph_t graph = nullptr;
+        cudaGraphConditionalHandle cond;
+        cudaGraphNode_t reset = nullptr, loop = nullptr;
+        cudaKernelNodeParams kp = {};
+        void* kargs[] = {&bw.loop};
+        kp.func = (void*)k_batch_loop_reset; kp.gridDim = dim3(1); kp.blockDim = dim3(1); kp.kernelParams = kargs;
+        cudaGraphNodeParams cp = {};
+        cp.type = cudaGraphNodeTypeConditional;
+        cp.conditional.type = cudaGraphCondTypeWhile; cp.conditional.size = 1;
+        cudaError_t ce = cudaGraphCreate(&graph, 0);
+        if (ce == cudaSuccess) ce = cudaGraphConditionalHandleCreate(&cond, graph, 1, cudaGraphCondAssignDefault);
+        if (ce == cudaSuccess) ce = cudaGraphAddKernelNode(&reset, graph, nullptr, 0, &kp);
+        if (ce == cudaSuccess) { cp.conditional.handle = cond; ce = cudaGraphAddNode(&loop, graph, &reset, 1, &cp); }
+        if (ce == cudaSuccess) ce = cudaStreamBeginCaptureToGraph(stream, cp.conditional.phGraph_out[0], nullptr, nullptr, 0,
+                                                                  cudaStreamCaptureModeRelaxed);
+        if (ce != cudaSuccess) {
+            if (graph) cudaGraphDestroy(graph);
+            set_error("building the batch loop graph failed: %s", cudaGetErrorString(ce));
+            return 2;
+        }
+        const int rc = fg(user, bw.nprob, bw.n, bw.x, bw.g, bw.f, bw.fgmask, (void*)stream);
+        if (bw.mt == 5) launch_dev_entry<5>();
+        else if (bw.mt == 10) launch_dev_entry<10>();
+        else launch_dev_entry<20>();
+        k_batch_loop_cond<<<1, 1, 0, stream>>>(cond, bw.loop, kLoopCallCap);
+        cudaGraph_t body = nullptr;
+        ce = cudaStreamEndCapture(stream, &body);
+        if (rc != 0 || ce != cudaSuccess) {
+            cudaGraphDestroy(graph);
+            cudaGetLastError();
+            set_error("the objective callback could not be captured in a CUDA graph (%s)", rc != 0 ? "callback failed" : cudaGetErrorString(ce));
+            return 1;
+        }
+        ce = cudaGraphInstantiate(&loop_exec, graph, 0);
+        cudaGraphDestroy(graph);
+        if (ce != cudaSuccess) { loop_exec = nullptr; set_error("cudaGraphInstantiate failed: %s", cudaGetErrorString(ce)); return 2; }
+        graph_builds++;
+        return 0;
+    }
+    // graph launches until no problem is at FG or NEW_X; then the state headers and the BS_* codes to the host
+    bool run_loop() {
+        const int P = bw.nprob;
+        CK(cudaMemsetAsync(bw.stop, 0, (size_t)P * sizeof(int), stream));
+        for (;;) {
+            CK(cudaGraphLaunch(loop_exec, stream));
+            graph_launches++;
+            CK(cudaMemcpyAsync(loop_host, bw.loop, 3 * sizeof(int), cudaMemcpyDeviceToHost, stream));
+            CK(cudaStreamSynchronize(stream));
+            graph_calls += loop_host[1];
+            if (loop_host[2] == 0) break;
+        }
+        CK(cudaMemcpy2DAsync(hdr_host, header_bytes, bw.s, sizeof(DevState<T>), header_bytes, P, cudaMemcpyDeviceToHost, stream));
+        CK(cudaMemcpyAsync(loop_host + 4, bw.stop, (size_t)P * sizeof(int), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        return true;
+    }
+    template <int MT> bool set_dev_attr() {
+        CK(cudaFuncSetAttribute(k_batch_setulb<T, MT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BatchSm<T>)));
+        return true;
+    }
+    // the loop's buffers, made at the first lbfgsb_batch_minimize_graph_* call of the handle
+    bool alloc_loop() {
+        if (!bw.loop && !dalloc(&bw.loop, 4 * sizeof(int))) return false;
+        if (!bw.stop && !dalloc(&bw.stop, (size_t)bw.nprob * sizeof(int))) return false;
+        CK(cudaMemsetAsync(bw.loop, 0, 4 * sizeof(int), stream));
+        if (!(bw.mt == 5 ? set_dev_attr<5>() : (bw.mt == 10 ? set_dev_attr<10>() : set_dev_attr<20>()))) return false;
+        CK(cudaMallocHost((void**)&loop_host, (4 + (size_t)bw.nprob) * sizeof(int)));
+        return true;
+    }
+    // Every problem from START to its end: START through call(), then graph launches of at most kLoopCallCap calls each
+    // while a problem is at FG or NEW_X, then one read-back of the state headers.  Returns 0, or 2 with the tasks of the
+    // problems that had not finished set to the failure (lbfgsb_b200_last_error has the reason).
+    template <typename FGE>
+    int minimize_graph(T* x, const T* l, const T* u, const int32_t* nbd, T* f, T* g, FGE fg, void* user, T factr, T pgtol,
+                       int32_t max_iter, int32_t max_fg, char* task, char* csave, int32_t* lsave, int32_t* isave, T* dsave) {
+        const int P = bw.nprob;
+        auto task_of = [&](int p) { return task + 60 * (size_t)p; };
+        std::vector<char> run(P, 0);
+        auto fail = [&](const char* text) {
+            for (int p = 0; p < P; ++p)
+                if (run[p]) { put60(task_of(p), text); started[p] = 2; }
+            n_fg = n_newx = 0; n_done = P;
+            return 2;
+        };
+        int drv = 0;
+        if (cudaDriverGetVersion(&drv) != cudaSuccess || drv < 12030) {
+            set_error("lbfgsb_batch_minimize_graph needs a CUDA 12.3 or later driver (conditional graph nodes); this one is %d.%d",
+                      drv / 1000, drv % 1000 / 10);
+            std::fill(run.begin(), run.end(), 1);
+            return fail("ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
+        }
+        for (int p = 0; p < P; ++p) put60(task_of(p), "START");
+        if (!call(x, l, u, nbd, f, g, factr, pgtol, task, csave, lsave, isave, dsave)) {
+            std::fill(run.begin(), run.end(), 1);
+            return fail("ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
+        }
+        graph_calls++;
+        if (n_fg == 0) return 0;
+        for (int p = 0; p < P; ++p) run[p] = pre60(task_of(p), "FG");
+        if (!loop_host && !alloc_loop()) return fail("ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
+        bw.max_iter = max_iter; bw.max_fg = max_fg;
+        LoopKey key;
+        memset(&key, 0, sizeof key);
+        key.x = x; key.l = l; key.u = u; key.nbd = nbd; key.f = f; key.g = g; key.fg = (void*)fg; key.user = user;
+        key.factr = factr; key.pgtol = pgtol; key.max_iter = max_iter; key.max_fg = max_fg;
+        if (!loop_exec || memcmp(&key, &loop_key, sizeof key) != 0) {
+            const int rc = build_loop_graph(fg, user);
+            if (rc != 0) {
+                memset(&loop_key, 0, sizeof loop_key);
+                cudaMemsetAsync(bw.fgmask, 0, (size_t)P * sizeof(int), stream);   // as the STOP call of solve leaves it
+                cudaStreamSynchronize(stream);
+                return fail(rc == 1 ? "STOP: THE OBJECTIVE CALLBACK FAILED" : "ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
+            }
+            loop_key = key;
+        }
+        if (!run_loop()) return fail("ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
+        const int* stop_host = loop_host + 4;
+        const double ph[3] = {0, 0, 0};
+        n_fg = n_newx = n_done = 0;
+        for (int p = 0; p < P; ++p) {
+            char* t = task_of(p);
+            if (run[p]) {
+                const DevState<T>* s = (const DevState<T>*)(hdr_host + (size_t)p * header_bytes);
+                export_state_of<T>(s, bw.n, ph, t, csave + 60 * (size_t)p, lsave + 4 * (size_t)p, isave + 44 * (size_t)p, dsave + 29 * (size_t)p);
+                if (stop_host[p]) {   // the caller's STOP of limit_stop: the problem is ended as by solve's STOP
+                    put60(t, stop_host[p] == BS_ITER ? "STOP: TOTAL NO. of ITERATIONS REACHED LIMIT" : "STOP: TOTAL NO. of f AND g EVALUATIONS EXCEEDS LIMIT");
+                    started[p] = 2;
+                }
+            }
+            if (pre60(t, "FG")) n_fg++;
+            else if (pre60(t, "NEW_X")) n_newx++;
+            else n_done++;
+        }
+        return 0;
+    }
 };
 
 // sample objective for a batch (test/driver1.f90:274-289, one CTA per problem): the arithmetic and the summation shape
@@ -2153,6 +2313,22 @@ __global__ void __launch_bounds__(LBFGSB_BLOCK) k_rosenbrock_batch(int nprob, i6
     }
     batch::final_sums<T>(1, n, sm, sm.red.rv);
     if (threadIdx.x == 0) f[p] = (T)4 * sm.red.rv[0];
+}
+
+// lbfgsb_batch_minimize_graph_*: the handle and kind check, then BatchEngine::minimize_graph
+template <typename T, typename FGE>
+static int batch_minimize_graph_impl(lbfgsb_batch_t* h, T* x, const T* l, const T* u, const int32_t* nbd, T* f, T* g, FGE fg, void* user,
+                                     T factr, T pgtol, int32_t max_iter, int32_t max_fg, char* task, char* csave, int32_t* lsave,
+                                     int32_t* isave, T* dsave) {
+    BatchBase* b = (BatchBase*)h;
+    if (!b || b->real_kind != (int)sizeof(T) || !fg) {
+        set_error(fg ? "invalid batch handle" : "no objective callback");
+        // every task of the handle's problems (of either kind), or the first one without a handle
+        const int P = !b ? 1 : (b->real_kind == 8 ? ((BatchEngine<double>*)b)->bw.nprob : ((BatchEngine<float>*)b)->bw.nprob);
+        if (task) for (int p = 0; p < P; ++p) put60(task + 60 * (size_t)p, "ERROR: INVALID LBFGSB_B200 HANDLE");
+        return 2;
+    }
+    return ((BatchEngine<T>*)b)->minimize_graph(x, l, u, nbd, f, g, fg, user, factr, pgtol, max_iter, max_fg, task, csave, lsave, isave, dsave);
 }
 
 // ---------------------------------------------------------------------------
@@ -2652,6 +2828,23 @@ void lbfgsb_batch_setulb_dev_f32(lbfgsb_batch_t* h, float* x, const float* l, co
     BatchEngine<float>* e = (BatchEngine<float>*)b;
     if (!e->call(x, l, u, nbd, f_dev, g, *factr, *pgtol, task, csave, lsave, isave, dsave))
         for (int p = 0; p < e->bw.nprob; ++p) put60(task + 60 * (size_t)p, "ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
+}
+int lbfgsb_batch_minimize_graph_f64(lbfgsb_batch_t* h, double* x, const double* l, const double* u, const int32_t* nbd, double* f_dev,
+                                    double* g, lbfgsb_batch_fg_enqueue_f64 fg, void* user, double factr, double pgtol, int32_t max_iter,
+                                    int32_t max_fg, char* task, char* csave, int32_t* lsave, int32_t* isave, double* dsave) {
+    return batch_minimize_graph_impl<double>(h, x, l, u, nbd, f_dev, g, fg, user, factr, pgtol, max_iter, max_fg, task, csave, lsave, isave, dsave);
+}
+int lbfgsb_batch_minimize_graph_f32(lbfgsb_batch_t* h, float* x, const float* l, const float* u, const int32_t* nbd, float* f_dev,
+                                    float* g, lbfgsb_batch_fg_enqueue_f32 fg, void* user, float factr, float pgtol, int32_t max_iter,
+                                    int32_t max_fg, char* task, char* csave, int32_t* lsave, int32_t* isave, float* dsave) {
+    return batch_minimize_graph_impl<float>(h, x, l, u, nbd, f_dev, g, fg, user, factr, pgtol, max_iter, max_fg, task, csave, lsave, isave, dsave);
+}
+int lbfgsb_batch_graph_stats(lbfgsb_batch_t* h, int64_t* graph_builds, int64_t* graph_launches, int64_t* calls) {
+    BatchBase* b = (BatchBase*)h;
+    if (!b || !graph_builds || !graph_launches || !calls) return 1;
+    if (b->real_kind == 8) { BatchEngine<double>* e = (BatchEngine<double>*)b; *graph_builds = e->graph_builds; *graph_launches = e->graph_launches; *calls = e->graph_calls; }
+    else { BatchEngine<float>* e = (BatchEngine<float>*)b; *graph_builds = e->graph_builds; *graph_launches = e->graph_launches; *calls = e->graph_calls; }
+    return 0;
 }
 int lbfgsb_batch_counts(lbfgsb_batch_t* h, int32_t* n_fg, int32_t* n_newx, int32_t* n_done) {
     BatchBase* b = (BatchBase*)h;
