@@ -274,7 +274,7 @@ __global__ void k_dw_adopt(Wk<T> w, const WalkCarry<T>* all, int turn, int R, in
     if (s->walk_J == LB_I64MAX) return;   // already closed by an earlier turn
     const WalkCarry<T>* cr = all + turn;
     const int col2 = 2 * s->col;
-    if (cr->found == 2) {   // redo the round up to the tie group, then the group in heap order (Engine::tie_replay_sharded)
+    if (cr->found == 2) {   // redo the round up to the tie group, then the group in heap order (Engine::tie_replay)
         s->tie_redo = 1; s->tie_key = cr->tie_key;
         s->walk_J = LB_I64MAX;   // the later turns of this round do nothing
         dc->jloc = 0;

@@ -114,11 +114,38 @@ __global__ void __launch_bounds__(256) k_publish(const unsigned* src, unsigned* 
     if (threadIdx.x == 0) { const unsigned long long v = *counter + 1; *counter = v; *flag_host = v; }
 }
 
-struct EngineBase {
-    virtual ~EngineBase() {}
+// What the handles of both engine families share: the real kind, and the device allocations freed with the handle.
+struct HandleBase {
+    virtual ~HandleBase() {}
     int real_kind;
+    std::vector<void*> allocs;
+    template <typename P> bool dalloc(P** p, size_t bytes) {
+        void* q = nullptr;
+        if (bytes == 0) bytes = 16;
+        cudaError_t e = cudaMalloc(&q, bytes);
+        if (e != cudaSuccess) { set_error("cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e)); return false; }
+        allocs.push_back(q);
+        *p = (P*)q;
+        return true;
+    }
+};
+struct EngineBase : HandleBase {
     lbprint::Ctx pr;     // the reference's text output (host_print.h)
 };
+// fn(E<double>*) or fn(E<float>*) with the engine behind handle b, by its real kind (E = Engine or BatchEngine)
+template <template <typename> class E, typename Fn>
+static auto with_kind(HandleBase* b, Fn fn) {
+    return b->real_kind == 8 ? fn((E<double>*)b) : fn((E<float>*)b);
+}
+// a new engine, or nullptr (lbfgsb_b200_last_error says why)
+template <typename E, typename... A>
+static E* new_engine(A... a) {
+    E* e = new E();
+    if (!e->init(a...)) { delete e; return nullptr; }
+    return e;
+}
+// the kernels' MT (common.cuh) for m corrections: 5, 10 or 20
+static int mt_of(int m) { return (m <= 5) ? 5 : (m <= 10 ? 10 : 20); }
 
 template <typename T>
 struct Engine : EngineBase {
@@ -138,7 +165,6 @@ struct Engine : EngineBase {
     SortCtl* ctl_host = nullptr;     // pinned
     T* tmpAB = nullptr; T* tmpF = nullptr; unsigned long long* jmin = nullptr;
     T* fd_parts = nullptr; T* delta = nullptr; T* delta_all = nullptr; T* delta_sum = nullptr;
-    std::vector<void*> allocs;
     // sharding
     int R = 1, rank = 0;
     ncclComm_t comm = nullptr;
@@ -231,20 +257,10 @@ struct Engine : EngineBase {
         return true;
     }
 
-    template <typename P> bool dalloc(P** p, size_t bytes) {
-        void* q = nullptr;
-        if (bytes == 0) bytes = 16;
-        cudaError_t e = cudaMalloc(&q, bytes);
-        if (e != cudaSuccess) { set_error("cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e)); return false; }
-        allocs.push_back(q);
-        *p = (P*)q;
-        return true;
-    }
-
     bool init(i64 n_, i64 off_, i64 ng_, int m_, cudaStream_t st, ncclComm_t cm, int rank_, int world_) {
         n = n_; offset = off_; n_global = ng_; m = m_; R = world_; rank = rank_; comm = cm;
         real_kind = (int)sizeof(T);
-        mt = (m <= 5) ? 5 : (m <= 10 ? 10 : 20);
+        mt = mt_of(m);
         fused = (mt == 5 ? fused_passes_ok<T, 5>() : (mt == 10 ? fused_passes_ok<T, 10>() : fused_passes_ok<T, 20>()));
         if (const char* e = getenv("LBFGSB_B200_NO_FUSION")) { if (e[0] == '1') fused = false; }
         fast = fused;   // the fast NEW_X pipeline is built from the fused passes
@@ -524,46 +540,11 @@ struct Engine : EngineBase {
         }
         return 0;
     }
-    // The exit fell inside the group of breakpoints equal to tie_key (single GPU): the round is redone up to
-    // that group, then the group runs as a round of its own in the reference's heap order (cauchy_walk.cuh
-    // "heap replay").  Returns like run_round.
+    // The exit fell inside the group of breakpoints equal to tie_key: the round is redone up to that group, then the group
+    // runs as a round of its own in the reference's heap order (cauchy_walk.cuh "heap replay").  Returns like run_round.
     int tie_replay(const BpRange& rg) {
-        if (R > 1) return tie_replay_sharded(rg);
         const unsigned long long tk = s_host->tie_key;
-        k_tie_restore<T><<<1, 32, 0, stream>>>(w); launches++;
-        if (tk > 0) {
-            BpRange ra = rg; ra.hi = tk - 1;
-            if (!(ra.lo_valid && ra.hi <= ra.lo)) {
-                const int st = run_round(ra);
-                if (st < 0) return -1;
-                if (st != 0) { set_error("heap replay: the round below the tie group did not pass (internal error)"); return -1; }
-            }
-        }
-        begin(F_WALK_COMPACT);
-        k_flag_count<T, 2><<<LG>>>(w, tile_counts);
-        k_tile_scan<T><<<1, 1024, 0, stream>>>(w, 2, tile_counts, tile_offsets, ntiles, wb.ctl);
-        k_flag_write<T, 2><<<LG>>>(w, tile_counts, tile_offsets, wb.k0, wb.v0);
-        end(F_WALK_COMPACT, 3);
-        if (s_host->nbreak <= LB_TIE_DEVICE_MAX) {
-            begin(F_WALK_SORT); k_heap_replay<T><<<1, 1024, 0, stream>>>(w, wb); end(F_WALK_SORT);
-        } else if (!heap_replay_on_host(tk)) return -1;
-        if (!sync_state()) return -1;
-        tie_replays++;
-        if (s_host->walk_lcount <= 0) { set_error("heap replay: empty tie group (internal error)"); return -1; }
-        if (!round_scan_single(s_host->walk_lcount)) return -1;
-        if (!sync_state()) return -1;
-        return s_host->walk_closed ? 1 : 0;
-    }
-    // The same on a sharded workspace.  The heap's history involves every breakpoint of the call, so every rank gathers
-    // all of them -- (t, global index), in variable order, exactly the reference's t / iorder arrays (:1305-1322) -- and
-    // pops the same heap on its host thread; the members of the group, in pop order, then form a round of their own whose
-    // sort keys are their positions in that order (tie_round = 2, walk_t_of): the sample sort, the exchange of the
-    // records and the scans in rank order run unchanged, and every rank fixes those of its own members that were passed.
-    DynBuf tie_k, tie_v, tie_kall, tie_vall;
-    int tie_replay_sharded(const BpRange& rg) {
-        typedef typename Real<T>::key_t K;
-        const unsigned long long tk = s_host->tie_key;
-        if (n_global >= 2147483647LL) { set_error("heap replay on a sharded workspace needs n < 2^31"); return -1; }
+        if (R > 1 && n_global >= 2147483647LL) { set_error("heap replay on a sharded workspace needs n < 2^31"); return -1; }
         k_tie_restore<T><<<1, 32, 0, stream>>>(w); launches++;
         if (tk > 0) {
             BpRange ra = rg; ra.hi = tk - 1;
@@ -579,65 +560,15 @@ struct Engine : EngineBase {
         k_tile_scan<T><<<1, 1024, 0, stream>>>(w, 2, tile_counts, tile_offsets, ntiles, wb.ctl);
         k_flag_write<T, 2><<<LG>>>(w, tile_counts, tile_offsets, wb.k0, wb.v0);
         end(F_WALK_COMPACT, 3);
-        SortCtl hc;
-        CK(cudaMemcpyAsync(&hc, wb.ctl, sizeof hc, cudaMemcpyDeviceToHost, stream));
-        CK(cudaStreamSynchronize(stream)); syncs++;
-        // counts and shard offsets of all ranks
-        RoundRec mine; mine.count = hc.count; mine.rem = offset; mine.kmin = 0; mine.pad = 0;
-        CK(cudaMemcpyAsync(rr_local, &mine, sizeof mine, cudaMemcpyHostToDevice, stream));
-        if (!allgather(rr_local, rr_all, sizeof(RoundRec))) return -1;
-        std::vector<RoundRec> recs((size_t)R);
-        CK(cudaMemcpyAsync(recs.data(), rr_all, sizeof(RoundRec) * R, cudaMemcpyDeviceToHost, stream));
-        CK(cudaStreamSynchronize(stream)); syncs++;
-        i64 maxc = 0, nb = 0;
-        for (int q = 0; q < R; ++q) { if (recs[q].count > maxc) maxc = recs[q].count; nb += recs[q].count; }
-        if (nb <= 0) { set_error("heap replay: no breakpoints (internal error)"); return -1; }
-        if (!ensure(tie_k, sizeof(K) * (size_t)maxc) || !ensure(tie_v, 4 * (size_t)maxc) ||
-            !ensure(tie_kall, sizeof(K) * (size_t)maxc * R) || !ensure(tie_vall, 4 * (size_t)maxc * R)) return -1;
-        CK(cudaMemcpyAsync(tie_k.p, wb.k0, sizeof(K) * (size_t)hc.count, cudaMemcpyDeviceToDevice, stream));
-        CK(cudaMemcpyAsync(tie_v.p, wb.v0, 4 * (size_t)hc.count, cudaMemcpyDeviceToDevice, stream));
-        if (!allgather(tie_k.p, tie_kall.p, sizeof(K) * (size_t)maxc) || !allgather(tie_v.p, tie_vall.p, 4 * (size_t)maxc)) return -1;
-        std::vector<K> hk((size_t)nb); std::vector<int> hv((size_t)nb);
-        {
-            i64 o = 0;
-            for (int q = 0; q < R; ++q) {
-                const i64 c = recs[q].count;
-                if (c > 0) {
-                    CK(cudaMemcpyAsync(hk.data() + o, (K*)tie_kall.p + (size_t)q * maxc, sizeof(K) * (size_t)c, cudaMemcpyDeviceToHost, stream));
-                    CK(cudaMemcpyAsync(hv.data() + o, (int*)tie_vall.p + (size_t)q * maxc, 4 * (size_t)c, cudaMemcpyDeviceToHost, stream));
-                }
-                o += c;
-            }
-            CK(cudaStreamSynchronize(stream)); syncs++;
-            o = 0;
-            for (int q = 0; q < R; ++q) {   // local -> global variable index (0-based); rem carries the shard offset
-                for (i64 i = 0; i < recs[q].count; ++i) hv[(size_t)(o + i)] += (int)recs[q].rem;
-                o += recs[q].count;
-            }
-        }
-        std::vector<K> gk; std::vector<int> gv;
-        heap_group_order((K)tk, hk, hv, (int)s_host->ibkmin, gk, gv);
-        // this rank's members: key = position in the pop order, value = local variable
-        std::vector<K> lk; std::vector<int> lv;
-        const i64 g = (i64)gv.size();
-        // REAL32: the position travels as a real in the exchanged record, exact below 2^24 -- a larger group is taken in
-        // variable order (what happens beyond the replay limit)
-        if (sizeof(T) == 4 && g >= ((i64)1 << 24)) std::sort(gv.begin(), gv.end());
-        for (i64 ppos = 0; ppos < g; ++ppos) {
-            const i64 gi = gv[(size_t)ppos];
-            if (gi >= offset && gi < offset + n) { lk.push_back((K)ppos); lv.push_back((int)(gi - offset)); }
-        }
-        const i64 cnt = (i64)lk.size();
-        if (cnt > 0) {
-            CK(cudaMemcpyAsync(wb.k1, lk.data(), sizeof(K) * (size_t)cnt, cudaMemcpyHostToDevice, stream));
-            CK(cudaMemcpyAsync(wb.v1, lv.data(), sizeof(int) * (size_t)cnt, cudaMemcpyHostToDevice, stream));
-        }
-        k_heap_replay_commit<T><<<1, 32, 0, stream>>>(w, wb, cnt, g, 2); launches++;
-        CK(cudaStreamSynchronize(stream));   // lk, lv are locals
+        i64 group = 0;   // the group's size over all ranks
+        if (R == 1 && s_host->nbreak <= LB_TIE_DEVICE_MAX) {
+            begin(F_WALK_SORT); k_heap_replay<T><<<1, 1024, 0, stream>>>(w, wb); end(F_WALK_SORT);
+        } else if (!heap_replay_on_host(tk, group)) return -1;
         if (!sync_state()) return -1;
         tie_replays++;
-        if (g <= 0) { set_error("heap replay: empty tie group (internal error)"); return -1; }
-        if (!round_scan_sharded()) return -1;
+        if (R == 1) group = s_host->walk_lcount;
+        if (group <= 0) { set_error("heap replay: empty tie group (internal error)"); return -1; }
+        if (R > 1 ? !round_scan_sharded() : !round_scan_single(s_host->walk_lcount)) return -1;
         if (!sync_state()) return -1;
         return s_host->walk_closed ? 1 : 0;
     }
@@ -662,27 +593,82 @@ struct Engine : EngineBase {
             if (out == tk) { gk.push_back(out); gv.push_back(var); }
         }
     }
-    // hpsolb's pop order of the group of breakpoints equal to tk, on the host (cauchy_walk.cuh "heap replay"): wb.k0 / wb.v0
-    // hold every breakpoint of this cauchy call in variable order.  The reference pays the same sequential heap.
-    bool heap_replay_on_host(unsigned long long tk64) {
+    // hpsolb's pop order of the group of breakpoints equal to tk on the host (long lists; cauchy_walk.cuh "heap replay"):
+    // wb.k0 / wb.v0 hold this rank's breakpoints of the cauchy call in variable order.  The reference pays the same
+    // sequential heap.  On one GPU the group goes to wb.k1 / wb.v1 as it is (keys = tk, tie_round = 1).  On a sharded
+    // workspace the heap's history involves every breakpoint of the call, so every rank gathers all of them -- (t, global
+    // index), in variable order, exactly the reference's t / iorder arrays (:1305-1322) -- and pops the same heap; its own
+    // members of the group, in pop order, then form a round whose sort keys are their positions in that order
+    // (tie_round = 2, walk_t_of): the sample sort, the exchange of the records and the scans in rank order run unchanged,
+    // and every rank fixes those of its own members that were passed.  `group` = the group's size over all ranks.
+    DynBuf tie_k, tie_v, tie_kall, tie_vall;
+    bool heap_replay_on_host(unsigned long long tk64, i64& group) {
         typedef typename Real<T>::key_t K;
         SortCtl hc;
         CK(cudaMemcpyAsync(&hc, wb.ctl, sizeof hc, cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream)); syncs++;
-        const i64 nb = hc.count;
-        if (nb <= 0) { set_error("heap replay: no breakpoints (internal error)"); return false; }
-        std::vector<K> hk((size_t)nb); std::vector<int> hv((size_t)nb);
-        CK(cudaMemcpyAsync(hk.data(), wb.k0, sizeof(K) * (size_t)nb, cudaMemcpyDeviceToHost, stream));
-        CK(cudaMemcpyAsync(hv.data(), wb.v0, sizeof(int) * (size_t)nb, cudaMemcpyDeviceToHost, stream));
-        CK(cudaStreamSynchronize(stream));
+        std::vector<K> hk; std::vector<int> hv;
+        if (R > 1) {
+            // counts and shard offsets of all ranks
+            RoundRec mine; mine.count = hc.count; mine.rem = offset; mine.kmin = 0; mine.pad = 0;
+            CK(cudaMemcpyAsync(rr_local, &mine, sizeof mine, cudaMemcpyHostToDevice, stream));
+            if (!allgather(rr_local, rr_all, sizeof(RoundRec))) return false;
+            std::vector<RoundRec> recs((size_t)R);
+            CK(cudaMemcpyAsync(recs.data(), rr_all, sizeof(RoundRec) * R, cudaMemcpyDeviceToHost, stream));
+            CK(cudaStreamSynchronize(stream)); syncs++;
+            i64 maxc = 0, nb = 0;
+            for (int q = 0; q < R; ++q) { if (recs[q].count > maxc) maxc = recs[q].count; nb += recs[q].count; }
+            if (nb <= 0) { set_error("heap replay: no breakpoints (internal error)"); return false; }
+            if (!ensure(tie_k, sizeof(K) * (size_t)maxc) || !ensure(tie_v, 4 * (size_t)maxc) ||
+                !ensure(tie_kall, sizeof(K) * (size_t)maxc * R) || !ensure(tie_vall, 4 * (size_t)maxc * R)) return false;
+            CK(cudaMemcpyAsync(tie_k.p, wb.k0, sizeof(K) * (size_t)hc.count, cudaMemcpyDeviceToDevice, stream));
+            CK(cudaMemcpyAsync(tie_v.p, wb.v0, 4 * (size_t)hc.count, cudaMemcpyDeviceToDevice, stream));
+            if (!allgather(tie_k.p, tie_kall.p, sizeof(K) * (size_t)maxc) || !allgather(tie_v.p, tie_vall.p, 4 * (size_t)maxc)) return false;
+            hk.resize((size_t)nb); hv.resize((size_t)nb);
+            i64 o = 0;
+            for (int q = 0; q < R; ++q) {
+                const i64 c = recs[q].count;
+                if (c > 0) {
+                    CK(cudaMemcpyAsync(hk.data() + o, (K*)tie_kall.p + (size_t)q * maxc, sizeof(K) * (size_t)c, cudaMemcpyDeviceToHost, stream));
+                    CK(cudaMemcpyAsync(hv.data() + o, (int*)tie_vall.p + (size_t)q * maxc, 4 * (size_t)c, cudaMemcpyDeviceToHost, stream));
+                }
+                o += c;
+            }
+            CK(cudaStreamSynchronize(stream)); syncs++;
+            o = 0;
+            for (int q = 0; q < R; ++q) {   // local -> global variable index (0-based); rem carries the shard offset
+                for (i64 i = 0; i < recs[q].count; ++i) hv[(size_t)(o + i)] += (int)recs[q].rem;
+                o += recs[q].count;
+            }
+        } else {
+            const i64 nb = hc.count;
+            if (nb <= 0) { set_error("heap replay: no breakpoints (internal error)"); return false; }
+            hk.resize((size_t)nb); hv.resize((size_t)nb);
+            CK(cudaMemcpyAsync(hk.data(), wb.k0, sizeof(K) * (size_t)nb, cudaMemcpyDeviceToHost, stream));
+            CK(cudaMemcpyAsync(hv.data(), wb.v0, sizeof(int) * (size_t)nb, cudaMemcpyDeviceToHost, stream));
+            CK(cudaStreamSynchronize(stream));
+        }
         std::vector<K> gk; std::vector<int> gv;
-        heap_group_order((K)tk64, hk, hv, (int)(s_host->ibkmin - offset), gk, gv);
+        heap_group_order((K)tk64, hk, hv, (int)(R > 1 ? s_host->ibkmin : s_host->ibkmin - offset), gk, gv);
+        group = (i64)gv.size();
+        if (R > 1) {
+            // this rank's members: key = position in the pop order, value = local variable.  REAL32: the position travels
+            // as a real in the exchanged record, exact below 2^24 -- a larger group is taken in variable order (what
+            // happens beyond the replay limit)
+            if (sizeof(T) == 4 && group >= ((i64)1 << 24)) std::sort(gv.begin(), gv.end());
+            std::vector<K> lk; std::vector<int> lv;
+            for (i64 ppos = 0; ppos < group; ++ppos) {
+                const i64 gi = gv[(size_t)ppos];
+                if (gi >= offset && gi < offset + n) { lk.push_back((K)ppos); lv.push_back((int)(gi - offset)); }
+            }
+            gk.swap(lk); gv.swap(lv);
+        }
         const i64 cnt = (i64)gk.size();
         if (cnt > 0) {
             CK(cudaMemcpyAsync(wb.k1, gk.data(), sizeof(K) * (size_t)cnt, cudaMemcpyHostToDevice, stream));
             CK(cudaMemcpyAsync(wb.v1, gv.data(), sizeof(int) * (size_t)cnt, cudaMemcpyHostToDevice, stream));
         }
-        k_heap_replay_commit<T><<<1, 32, 0, stream>>>(w, wb, cnt, cnt, 1); launches++;
+        k_heap_replay_commit<T><<<1, 32, 0, stream>>>(w, wb, cnt, group, R > 1 ? 2 : 1); launches++;
         CK(cudaStreamSynchronize(stream));   // gk, gv are locals
         return true;
     }
@@ -719,23 +705,31 @@ struct Engine : EngineBase {
         if (!s_host->walk_closed) { set_error("the breakpoint walk did not close (internal error)"); return false; }
         return true;
     }
+    // The scans of a sorted list of `count` breakpoints in wd, one chunk of at most wd.cap after another.  A chunk's
+    // records are gathered from the workspace (k_walk_gather), or, given `recv`, from the exchanged records of rs reals
+    // each (k_dw_gather).
+    bool scan_chunks(const WalkBuf<T>& wd, i64 count, const T* recv = nullptr, int rs = 0) {
+        for (i64 start = 0; start < count; start += wd.cap) {
+            const i64 len = (count - start < wd.cap) ? (count - start) : wd.cap;
+            const i64 nblk = (len + LB_WB - 1) / LB_WB;
+            CK(cudaMemsetAsync(jmin, 0xff, 8, stream));
+            if (recv) k_dw_gather<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, recv, rs, start, len);
+            else k_walk_gather<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
+            k_walk_scan_vec<T><<<1, 1024, 0, stream>>>(w, wd, nblk, tmpAB);
+            k_walk_dots<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
+            k_walk_scan_f2<T><<<1, 32, 0, stream>>>(w, wd, nblk, tmpF);
+            k_walk_f2<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
+            k_walk_scan_f1<T><<<1, 32, 0, stream>>>(w, wd, nblk, tmpF);
+            k_walk_test<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len, jmin);
+            k_walk_chunk_end<T><<<1, 32, 0, stream>>>(w, wd, start, len, tmpAB, tmpF, jmin);
+            launches += 8;
+        }
+        return true;
+    }
     // scans of one round's sorted list on a single GPU
     bool round_scan_single(i64 count) {
         begin(F_WALK_SCAN);
-        for (i64 start = 0; start < count; start += wb.cap) {
-            const i64 len = (count - start < wb.cap) ? (count - start) : wb.cap;
-            const i64 nblk = (len + LB_WB - 1) / LB_WB;
-            CK(cudaMemsetAsync(jmin, 0xff, 8, stream));
-            k_walk_gather<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wb, start, len);
-            k_walk_scan_vec<T><<<1, 1024, 0, stream>>>(w, wb, nblk, tmpAB);
-            k_walk_dots<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wb, start, len);
-            k_walk_scan_f2<T><<<1, 32, 0, stream>>>(w, wb, nblk, tmpF);
-            k_walk_f2<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wb, start, len);
-            k_walk_scan_f1<T><<<1, 32, 0, stream>>>(w, wb, nblk, tmpF);
-            k_walk_test<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wb, start, len, jmin);
-            k_walk_chunk_end<T><<<1, 32, 0, stream>>>(w, wb, start, len, tmpAB, tmpF, jmin);
-            launches += 8;
-        }
+        if (!scan_chunks(wb, count)) return false;
         k_walk_round_end<T><<<1, LB_WB, 0, stream>>>(w, wb, n_global, R == 1 ? 1 : 0);
         end(F_WALK_SCAN, 1);
         begin(F_WALK_FIX);
@@ -781,39 +775,32 @@ struct Engine : EngineBase {
             launches += 4;
         }
     }
+    // wd = wb with the sort buffers of an exchanged list of `count` breakpoints and its own sort control
+    bool exchanged_buf(i64 count, WalkBuf<T>& wd) {
+        typedef typename Real<T>::key_t K;
+        if (!ensure(dw_k0, sizeof(K) * (size_t)count) || !ensure(dw_k1, sizeof(K) * (size_t)count) ||
+            !ensure(dw_v0, 4 * (size_t)count) || !ensure(dw_v1, 4 * (size_t)count)) return false;
+        wd = wb;
+        wd.k0 = (K*)dw_k0.p; wd.k1 = (K*)dw_k1.p; wd.v0 = (int*)dw_v0.p; wd.v1 = (int*)dw_v1.p; wd.ctl = ctl_d;
+        return true;
+    }
     // a small round on a sharded problem (cauchy_walk_dist.cuh "Small rounds"): every rank scans the whole gathered list
     bool round_scan_gathered(i64 total) {
-        typedef typename Real<T>::key_t K;
         const int col = s_host->col;
         const int rs = 3 + 2 * col;
         const i64 cap = (total + 63) / 64 * 64;   // >= every rank's count of the round
         if (!ensure(dw_send, sizeof(T) * (size_t)cap * rs) || !ensure(dw_recv, sizeof(T) * (size_t)cap * rs * R)) return false;
-        if (!ensure(dw_k0, sizeof(K) * (size_t)total) || !ensure(dw_k1, sizeof(K) * (size_t)total) ||
-            !ensure(dw_v0, 4 * (size_t)total) || !ensure(dw_v1, 4 * (size_t)total)) return false;
+        WalkBuf<T> wd;
+        if (!exchanged_buf(total, wd)) return false;
         begin(F_WALK_SCAN);
         k_rw_count<T><<<1, 32, 0, stream>>>(w, wb, rr_local); launches++;
         if (!allgather(rr_local, rr_all, sizeof(RoundRec))) return false;
         T* send = (T*)dw_send.p; T* recv = (T*)dw_recv.p;
         k_dw_pack<T><<<LBFGSB_GRID, 256, 0, stream>>>(w, wb, send, rs); launches++;
         if (!allgather(send, recv, sizeof(T) * (size_t)cap * rs)) return false;
-        WalkBuf<T> wd = wb;
-        wd.k0 = (K*)dw_k0.p; wd.k1 = (K*)dw_k1.p; wd.v0 = (int*)dw_v0.p; wd.v1 = (int*)dw_v1.p; wd.ctl = ctl_d;
         k_rw_keys<T><<<32, 256, 0, stream>>>(recv, rs, cap, rr_all, R, wd.k0, wd.v0, ctl_d); launches++;
         enqueue_sort(wd.k0, wd.k1, wd.v0, wd.v1, ctl_d, total);
-        for (i64 start = 0; start < total; start += wd.cap) {
-            const i64 len = (total - start < wd.cap) ? (total - start) : wd.cap;
-            const i64 nblk = (len + LB_WB - 1) / LB_WB;
-            CK(cudaMemsetAsync(jmin, 0xff, 8, stream));
-            k_dw_gather<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, recv, rs, start, len);
-            k_walk_scan_vec<T><<<1, 1024, 0, stream>>>(w, wd, nblk, tmpAB);
-            k_walk_dots<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
-            k_walk_scan_f2<T><<<1, 32, 0, stream>>>(w, wd, nblk, tmpF);
-            k_walk_f2<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
-            k_walk_scan_f1<T><<<1, 32, 0, stream>>>(w, wd, nblk, tmpF);
-            k_walk_test<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len, jmin);
-            k_walk_chunk_end<T><<<1, 32, 0, stream>>>(w, wd, start, len, tmpAB, tmpF, jmin);
-            launches += 8;
-        }
+        if (!scan_chunks(wd, total, recv, rs)) return false;
         k_walk_round_end<T><<<1, LB_WB, 0, stream>>>(w, wd, n_global, 1);
         end(F_WALK_SCAN, 1);
         begin(F_WALK_FIX);
@@ -823,7 +810,6 @@ struct Engine : EngineBase {
     }
     // one round on a sharded problem: this rank's breakpoints of the round are sorted in wb
     bool round_scan_sharded() {
-        typedef typename Real<T>::key_t K;
         if (s_host->walk_rcount > 0 && s_host->walk_rcount <= LB_RW_MAX) return round_scan_gathered(s_host->walk_rcount);
         const int S = LB_DW_SAMPLES;
         // 2. splitters from regular samples
@@ -866,8 +852,8 @@ struct Engine : EngineBase {
         const int col = s_host->col;
         const int rs = 3 + 2 * col;
         if (!ensure(dw_send, sizeof(T) * (size_t)nb_loc * rs) || !ensure(dw_recv, sizeof(T) * (size_t)nrecv * rs)) return false;
-        if (!ensure(dw_k0, sizeof(K) * (size_t)nrecv) || !ensure(dw_k1, sizeof(K) * (size_t)nrecv) ||
-            !ensure(dw_v0, 4 * (size_t)nrecv) || !ensure(dw_v1, 4 * (size_t)nrecv)) return false;
+        WalkBuf<T> wd;
+        if (!exchanged_buf(nrecv, wd)) return false;
         CK(cudaMemcpyAsync(dctl, &hc, sizeof hc, cudaMemcpyHostToDevice, stream));
         CK(cudaStreamSynchronize(stream));   // hc is a stack object
         T* send = (T*)dw_send.p; T* recv = (T*)dw_recv.p;
@@ -885,27 +871,12 @@ struct Engine : EngineBase {
         int grc = nccl_api()->GroupEnd();
         if (grc != 0) { set_error("nccl send/recv group failed: %d", grc); return false; }
         // 4. this rank's key range in global order
-        WalkBuf<T> wd = wb;
-        wd.k0 = (K*)dw_k0.p; wd.k1 = (K*)dw_k1.p; wd.v0 = (int*)dw_v0.p; wd.v1 = (int*)dw_v1.p; wd.ctl = ctl_d;
         k_dw_keys<T><<<LBFGSB_GRID, 256, 0, stream>>>(recv, rs, nrecv, wd.k0, wd.v0, ctl_d); launches++;
         enqueue_sort(wd.k0, wd.k1, wd.v0, wd.v1, ctl_d, nrecv);
         // 5. scans in rank order, carries handed from rank to rank
         for (int turn = 0; turn < R; ++turn) {
             if (turn == rank) {
-                for (i64 start = 0; start < nrecv; start += wd.cap) {
-                    const i64 len = (nrecv - start < wd.cap) ? (nrecv - start) : wd.cap;
-                    const i64 nblk = (len + LB_WB - 1) / LB_WB;
-                    CK(cudaMemsetAsync(jmin, 0xff, 8, stream));
-                    k_dw_gather<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, recv, rs, start, len);
-                    k_walk_scan_vec<T><<<1, 1024, 0, stream>>>(w, wd, nblk, tmpAB);
-                    k_walk_dots<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
-                    k_walk_scan_f2<T><<<1, 32, 0, stream>>>(w, wd, nblk, tmpF);
-                    k_walk_f2<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len);
-                    k_walk_scan_f1<T><<<1, 32, 0, stream>>>(w, wd, nblk, tmpF);
-                    k_walk_test<T><<<(unsigned)nblk, LB_WB, 0, stream>>>(w, wd, start, len, jmin);
-                    k_walk_chunk_end<T><<<1, 32, 0, stream>>>(w, wd, start, len, tmpAB, tmpF, jmin);
-                    launches += 8;
-                }
+                if (!scan_chunks(wd, nrecv, recv, rs)) return false;
                 k_dw_fixcount<T><<<LBFGSB_GRID, 256, 0, stream>>>(w, wd, R, dctl); launches++;
             }
             k_dw_turn_end<T><<<1, LB_WB, 0, stream>>>(w, wd, dctl, wd.cap, turn == rank ? 1 : 0, R, carry_local); launches++;
@@ -1478,17 +1449,20 @@ static int task_return_code(const char* task) {
     if (pre60(task, "ABNO")) return 1;
     return 2;
 }
-template <typename T, typename FG>
-static int minimize_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, const int32_t* nbd, FG fg, void* user, T factr, T pgtol,
+// One loop for both: FG -> `eval` (false: the callback failed, the loop STOPs), NEW_X -> the caller's limits, any other task
+// ends it.  `takeover(e)` runs after every setulb call and may advance the state itself; false from it is a CUDA failure.
+template <typename T, typename Eval, typename Takeover>
+static int minimize_loop(lbfgsb_dev_t* h, bool has_fg, T* x, const T* l, const T* u, const int32_t* nbd, T factr, T pgtol,
                          int32_t max_iter, int32_t max_fg, int32_t iprint, T* f, T* g, char* task, char* csave, int32_t* lsave,
-                         int32_t* isave, T* dsave) {
+                         int32_t* isave, T* dsave, Eval eval, Takeover takeover) {
     Engine<T>* e = (Engine<T>*)h;
-    if (!e || e->real_kind != (int)sizeof(T) || !fg) { put60(task, "ERROR: INVALID LBFGSB_B200 HANDLE"); return 2; }
+    if (!e || e->real_kind != (int)sizeof(T) || !has_fg) { put60(task, "ERROR: INVALID LBFGSB_B200 HANDLE"); return 2; }
     put60(task, "START");
     for (;;) {
         setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
+        if (!takeover(e)) return 2;
         if (pre60(task, "FG")) {
-            if (fg(user, e->n, x, g, f, (void*)e->stream) != 0) {
+            if (!eval(e)) {
                 put60(task, "STOP: THE OBJECTIVE CALLBACK FAILED");
                 setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
                 return 2;
@@ -1502,6 +1476,14 @@ static int minimize_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, const in
         } else return task_return_code(task);
     }
 }
+template <typename T, typename FG>
+static int minimize_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, const int32_t* nbd, FG fg, void* user, T factr, T pgtol,
+                         int32_t max_iter, int32_t max_fg, int32_t iprint, T* f, T* g, char* task, char* csave, int32_t* lsave,
+                         int32_t* isave, T* dsave) {
+    return minimize_loop<T>(h, fg != nullptr, x, l, u, nbd, factr, pgtol, max_iter, max_fg, iprint, f, g, task, csave, lsave, isave, dsave,
+                            [&](Engine<T>* e) { return fg(user, e->n, x, g, f, (void*)e->stream) == 0; },
+                            [](Engine<T>*) { return true; });
+}
 
 // The same loop kept on the device: the objective callback only ENQUEUES work on the given stream and leaves f in device
 // memory, so that one iteration step -- objective, FG_LNSRCH entry, NEW_X entry -- is captured once as a CUDA graph and
@@ -1511,48 +1493,32 @@ template <typename T, typename FGE>
 static int minimize_graph_impl(lbfgsb_dev_t* h, T* x, const T* l, const T* u, const int32_t* nbd, FGE fg, void* user, T factr, T pgtol,
                                int32_t max_iter, int32_t max_fg, T* f, T* g, char* task, char* csave, int32_t* lsave,
                                int32_t* isave, T* dsave) {
-    Engine<T>* e = (Engine<T>*)h;
-    if (!e || e->real_kind != (int)sizeof(T) || !fg) { put60(task, "ERROR: INVALID LBFGSB_B200 HANDLE"); return 2; }
-    const int32_t iprint = -1;
-    auto eval_host = [&]() -> bool {   // one evaluation outside the graph: f comes back to the host
+    auto eval_host = [&](Engine<T>* e) -> bool {   // one evaluation outside the graph: f comes back to the host
         if (fg(user, e->n, x, g, e->f_dev, (void*)e->stream) != 0) return false;
         if (cudaMemcpyAsync(f, e->f_dev, sizeof(T), cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) return false;
         return cudaStreamSynchronize(e->stream) == cudaSuccess;
     };
-    put60(task, "START");
     bool graph_ok = false, graph_tried = false;
-    for (;;) {
-        setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
-        // the device-resident loop takes over whenever the state asks for a line-search evaluation
-        if (pre60(task, "FG_LN") && e->fast && e->R == 1 && e->s_host->cnstnd) {
-            if (!graph_tried) {
-                graph_tried = true;
-                e->w.x = x; e->w.l = l; e->w.u = u; e->w.nbd = nbd; e->w.g = g;
-                graph_ok = e->build_iter_graph(fg, user, max_iter, max_fg);
-            }
-            if (graph_ok) {
-                e->w.x = x; e->w.l = l; e->w.u = u; e->w.nbd = nbd; e->w.g = g; e->w.bp_hint = 0;
-                bool ok = true;
-                while (ok && e->s_host->task == TK_FG_LNSRCH) ok = e->graph_step();
-                if (!ok) { put60(task, "ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)"); return 2; }
-                *f = e->s_host->f;
-                export_state<T>(e, task, csave, lsave, isave, dsave);
-            }
+    // the device-resident loop takes over whenever the state asks for a line-search evaluation
+    auto graph_loop = [&](Engine<T>* e) -> bool {
+        if (!(pre60(task, "FG_LN") && e->fast && e->R == 1 && e->s_host->cnstnd)) return true;
+        if (!graph_tried) {
+            graph_tried = true;
+            e->w.x = x; e->w.l = l; e->w.u = u; e->w.nbd = nbd; e->w.g = g;
+            graph_ok = e->build_iter_graph(fg, user, max_iter, max_fg);
         }
-        if (pre60(task, "FG")) {
-            if (!eval_host()) {
-                put60(task, "STOP: THE OBJECTIVE CALLBACK FAILED");
-                setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
-                return 2;
-            }
-        } else if (pre60(task, "NEW_X")) {
-            if (const char* stop = limit_stop(isave, max_iter, max_fg)) {
-                put60(task, stop);
-                setulb_dev_impl<T>(h, x, l, u, nbd, f, g, &factr, &pgtol, task, &iprint, csave, lsave, isave, dsave);
-                return 0;
-            }
-        } else return task_return_code(task);
-    }
+        if (graph_ok) {
+            e->w.x = x; e->w.l = l; e->w.u = u; e->w.nbd = nbd; e->w.g = g; e->w.bp_hint = 0;
+            bool ok = true;
+            while (ok && e->s_host->task == TK_FG_LNSRCH) ok = e->graph_step();
+            if (!ok) { put60(task, "ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)"); return false; }
+            *f = e->s_host->f;
+            export_state<T>(e, task, csave, lsave, isave, dsave);
+        }
+        return true;
+    };
+    return minimize_loop<T>(h, fg != nullptr, x, l, u, nbd, factr, pgtol, max_iter, max_fg, -1, f, g, task, csave, lsave, isave, dsave,
+                            eval_host, graph_loop);
 }
 
 // ---------------------------------------------------------------------------
@@ -1983,39 +1949,39 @@ static TrialSums<T> trial_sums_of(Engine<T>* e, const T* l, const T* u, const in
 // ---------------------------------------------------------------------------
 // Batched small problems (batch.cuh; include/lbfgsb_b200.h section 6)
 // ---------------------------------------------------------------------------
-struct BatchBase {
-    virtual ~BatchBase() {}
-    int real_kind;
-};
 template <typename T>
-struct BatchEngine : BatchBase {
+struct BatchEngine : HandleBase {
     BatchWk<T> bw;
     cudaStream_t stream = 0;
     bool own_stream = false;
-    std::vector<void*> allocs;
     int* entry_dev = nullptr; int* entry_host = nullptr;
     char* hdr_host = nullptr;          // [nprob][header_bytes], pinned
     size_t header_bytes = 0;
     std::vector<char> started;
     int n_fg = 0, n_newx = 0, n_done = 0;
     i64 launches = 0;
-    template <typename P> bool dalloc(P** p, size_t bytes) {
-        void* q = nullptr;
-        if (bytes == 0) bytes = 16;
-        cudaError_t e = cudaMalloc(&q, bytes);
-        if (e != cudaSuccess) { set_error("cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e)); return false; }
-        allocs.push_back(q);
-        *p = (P*)q;
-        return true;
+    // k_batch_setulb for the handle's MT; DEV: the entry of the task loop on the device
+    template <bool DEV> auto setulb_kernel() const {
+        if (bw.mt == 5) return k_batch_setulb<T, 5, DEV>;
+        if (bw.mt == 10) return k_batch_setulb<T, 10, DEV>;
+        return k_batch_setulb<T, 20, DEV>;
     }
-    template <int MT> bool set_attr() {
-        CK(cudaFuncSetAttribute(k_batch_setulb<T, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BatchSm<T>)));
-        return true;
+    const DevState<T>* header(int p) const { return (const DevState<T>*)(hdr_host + (size_t)p * header_bytes); }
+    // problem p's state header -> its slices of the caller's task / csave / lsave / isave / dsave
+    void export_problem(int p, char* task, char* csave, int32_t* lsave, int32_t* isave, T* dsave) const {
+        const double ph[3] = {0, 0, 0};
+        const size_t q = (size_t)p;
+        export_state_of<T>(header(p), bw.n, ph, task + 60 * q, csave + 60 * q, lsave + 4 * q, isave + 44 * q, dsave + 29 * q);
+    }
+    void tally(const char* t) {
+        if (pre60(t, "FG")) n_fg++;
+        else if (pre60(t, "NEW_X")) n_newx++;
+        else n_done++;
     }
     bool init(int nprob, i64 n, int m, cudaStream_t st) {
         real_kind = (int)sizeof(T);
         memset(&bw, 0, sizeof bw);
-        bw.nprob = nprob; bw.n = n; bw.m = m; bw.mt = (m <= 5) ? 5 : (m <= 10 ? 10 : 20);
+        bw.nprob = nprob; bw.n = n; bw.m = m; bw.mt = mt_of(m);
         bw.ldw = (n + 31) / 32 * 32;
         if (st) stream = st;
         else { CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking)); own_stream = true; }
@@ -2035,7 +2001,7 @@ struct BatchEngine : BatchBase {
         CK(cudaMallocHost((void**)&hdr_host, P * header_bytes));
         CK(cudaMallocHost((void**)&entry_host, P * sizeof(int)));
         started.assign(P, 0);
-        if (!(bw.mt == 5 ? set_attr<5>() : (bw.mt == 10 ? set_attr<10>() : set_attr<20>()))) return false;
+        CK(cudaFuncSetAttribute(setulb_kernel<false>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BatchSm<T>)));
         CK(cudaStreamSynchronize(stream));
         return true;
     }
@@ -2071,31 +2037,24 @@ struct BatchEngine : BatchBase {
             bw.x = x; bw.l = l; bw.u = u; bw.nbd = nbd; bw.g = g; bw.f = f; bw.factr = factr; bw.pgtol = pgtol;
             bw.entry = entry_dev;
             CK(cudaMemcpyAsync(entry_dev, entry_host, sizeof(int) * P, cudaMemcpyHostToDevice, stream));
-            const size_t smem = sizeof(BatchSm<T>);
-            if (bw.mt == 5) k_batch_setulb<T, 5><<<P, LBFGSB_BLOCK, smem, stream>>>(bw);
-            else if (bw.mt == 10) k_batch_setulb<T, 10><<<P, LBFGSB_BLOCK, smem, stream>>>(bw);
-            else k_batch_setulb<T, 20><<<P, LBFGSB_BLOCK, smem, stream>>>(bw);
+            setulb_kernel<false>()<<<P, LBFGSB_BLOCK, sizeof(BatchSm<T>), stream>>>(bw);
             launches++;
             CK(cudaMemcpy2DAsync(hdr_host, header_bytes, bw.s, sizeof(DevState<T>), header_bytes, P, cudaMemcpyDeviceToHost, stream));
             CK(cudaStreamSynchronize(stream));
             cudaError_t le = cudaGetLastError();
             if (le != cudaSuccess) { set_error("batch kernel failed: %s", cudaGetErrorString(le)); return false; }
         }
-        const double ph[3] = {0, 0, 0};
         for (int p = 0; p < P; ++p) {
             char* t = task + 60 * (size_t)p;
             const int e = entry_host[p];
             if (e != BE_IDLE) {
-                const DevState<T>* s = (const DevState<T>*)(hdr_host + (size_t)p * header_bytes);
                 if (e == BE_STOP_CPU) { /* the caller's STOP text stays in task; x, g, f were restored */ }
                 else {
-                    export_state_of<T>(s, bw.n, ph, t, csave + 60 * (size_t)p, lsave + 4 * (size_t)p, isave + 44 * (size_t)p, dsave + 29 * (size_t)p);
-                    if (e == BE_START && pre60(t, "ERROR")) { isave[44 * (size_t)p + 34] = s->info; isave[44 * (size_t)p + 41] = (int32_t)s->errk; }
+                    export_problem(p, task, csave, lsave, isave, dsave);
+                    if (e == BE_START && pre60(t, "ERROR")) { isave[44 * (size_t)p + 34] = header(p)->info; isave[44 * (size_t)p + 41] = (int32_t)header(p)->errk; }
                 }
             }
-            if (pre60(t, "FG")) n_fg++;
-            else if (pre60(t, "NEW_X")) n_newx++;
-            else n_done++;
+            tally(t);
         }
         return true;
     }
@@ -2137,9 +2096,6 @@ struct BatchEngine : BatchBase {
     int* loop_host = nullptr;                  // pinned [4 + nprob]: loop[0..2] of the device, then the BS_* codes
     i64 graph_builds = 0, graph_launches = 0, graph_calls = 0;
 
-    template <int MT> void launch_dev_entry() {
-        k_batch_setulb<T, MT, true><<<bw.nprob, LBFGSB_BLOCK, sizeof(BatchSm<T>), stream>>>(bw);
-    }
     // 0 built; 1 the objective failed or could not be captured; 2 CUDA failure
     template <typename FGE>
     int build_loop_graph(FGE fg, void* user) {
@@ -2165,9 +2121,7 @@ struct BatchEngine : BatchBase {
             return 2;
         }
         const int rc = fg(user, bw.nprob, bw.n, bw.x, bw.g, bw.f, bw.fgmask, (void*)stream);
-        if (bw.mt == 5) launch_dev_entry<5>();
-        else if (bw.mt == 10) launch_dev_entry<10>();
-        else launch_dev_entry<20>();
+        setulb_kernel<true>()<<<bw.nprob, LBFGSB_BLOCK, sizeof(BatchSm<T>), stream>>>(bw);
         k_batch_loop_cond<<<1, 1, 0, stream>>>(cond, bw.loop, kLoopCallCap);
         cudaGraph_t body = nullptr;
         ce = cudaStreamEndCapture(stream, &body);
@@ -2200,16 +2154,12 @@ struct BatchEngine : BatchBase {
         CK(cudaStreamSynchronize(stream));
         return true;
     }
-    template <int MT> bool set_dev_attr() {
-        CK(cudaFuncSetAttribute(k_batch_setulb<T, MT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BatchSm<T>)));
-        return true;
-    }
     // the loop's buffers, made at the first lbfgsb_batch_minimize_graph_* call of the handle
     bool alloc_loop() {
         if (!bw.loop && !dalloc(&bw.loop, 4 * sizeof(int))) return false;
         if (!bw.stop && !dalloc(&bw.stop, (size_t)bw.nprob * sizeof(int))) return false;
         CK(cudaMemsetAsync(bw.loop, 0, 4 * sizeof(int), stream));
-        if (!(bw.mt == 5 ? set_dev_attr<5>() : (bw.mt == 10 ? set_dev_attr<10>() : set_dev_attr<20>()))) return false;
+        CK(cudaFuncSetAttribute(setulb_kernel<true>(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BatchSm<T>)));
         CK(cudaMallocHost((void**)&loop_host, (4 + (size_t)bw.nprob) * sizeof(int)));
         return true;
     }
@@ -2261,21 +2211,17 @@ struct BatchEngine : BatchBase {
         }
         if (!run_loop()) return fail("ERROR: CUDA FAILURE (see lbfgsb_b200_last_error)");
         const int* stop_host = loop_host + 4;
-        const double ph[3] = {0, 0, 0};
         n_fg = n_newx = n_done = 0;
         for (int p = 0; p < P; ++p) {
             char* t = task_of(p);
             if (run[p]) {
-                const DevState<T>* s = (const DevState<T>*)(hdr_host + (size_t)p * header_bytes);
-                export_state_of<T>(s, bw.n, ph, t, csave + 60 * (size_t)p, lsave + 4 * (size_t)p, isave + 44 * (size_t)p, dsave + 29 * (size_t)p);
+                export_problem(p, task, csave, lsave, isave, dsave);
                 if (stop_host[p]) {   // the caller's STOP of limit_stop: the problem is ended as by solve's STOP
                     put60(t, stop_host[p] == BS_ITER ? "STOP: TOTAL NO. of ITERATIONS REACHED LIMIT" : "STOP: TOTAL NO. of f AND g EVALUATIONS EXCEEDS LIMIT");
                     started[p] = 2;
                 }
             }
-            if (pre60(t, "FG")) n_fg++;
-            else if (pre60(t, "NEW_X")) n_newx++;
-            else n_done++;
+            tally(t);
         }
         return 0;
     }
@@ -2320,11 +2266,11 @@ template <typename T, typename FGE>
 static int batch_minimize_graph_impl(lbfgsb_batch_t* h, T* x, const T* l, const T* u, const int32_t* nbd, T* f, T* g, FGE fg, void* user,
                                      T factr, T pgtol, int32_t max_iter, int32_t max_fg, char* task, char* csave, int32_t* lsave,
                                      int32_t* isave, T* dsave) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b || b->real_kind != (int)sizeof(T) || !fg) {
         set_error(fg ? "invalid batch handle" : "no objective callback");
         // every task of the handle's problems (of either kind), or the first one without a handle
-        const int P = !b ? 1 : (b->real_kind == 8 ? ((BatchEngine<double>*)b)->bw.nprob : ((BatchEngine<float>*)b)->bw.nprob);
+        const int P = !b ? 1 : with_kind<BatchEngine>(b, [](auto* e) { return e->bw.nprob; });
         if (task) for (int p = 0; p < P; ++p) put60(task + 60 * (size_t)p, "ERROR: INVALID LBFGSB_B200 HANDLE");
         return 2;
     }
@@ -2375,15 +2321,10 @@ lbfgsb_dev_t* lbfgsb_dev_create_sharded(int64_t n_local, int64_t offset, int64_t
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { set_error("no CUDA device (lbfgsb_b200 has no CPU path)"); return nullptr; }
     if (world > 1 && (!nccl_comm || !nccl_api()->ok)) { set_error("sharded engine needs an NCCL communicator"); return nullptr; }
-    if (real_kind == 8) {
-        Engine<double>* e = new Engine<double>();
-        if (!e->init(n_local, offset, n_global, m, (cudaStream_t)cuda_stream, (ncclComm_t)nccl_comm, rank, world)) { delete e; return nullptr; }
-        return (lbfgsb_dev_t*)e;
-    } else if (real_kind == 4) {
-        Engine<float>* e = new Engine<float>();
-        if (!e->init(n_local, offset, n_global, m, (cudaStream_t)cuda_stream, (ncclComm_t)nccl_comm, rank, world)) { delete e; return nullptr; }
-        return (lbfgsb_dev_t*)e;
-    }
+    if (real_kind == 8)
+        return (lbfgsb_dev_t*)new_engine<Engine<double>>(n_local, offset, n_global, m, (cudaStream_t)cuda_stream, (ncclComm_t)nccl_comm, rank, world);
+    if (real_kind == 4)
+        return (lbfgsb_dev_t*)new_engine<Engine<float>>(n_local, offset, n_global, m, (cudaStream_t)cuda_stream, (ncclComm_t)nccl_comm, rank, world);
     set_error("real_kind must be 8 or 4");
     return nullptr;
 }
@@ -2447,13 +2388,13 @@ int lbfgsb_dev_checkpoint_write(lbfgsb_dev_t* h, const char* path) {
     EngineBase* b = (EngineBase*)h;
     if (!b || !path) return 1;
     g_last_error.clear();
-    return ((b->real_kind == 8) ? ((Engine<double>*)b)->checkpoint_io(path, true) : ((Engine<float>*)b)->checkpoint_io(path, true)) ? 0 : 1;
+    return with_kind<Engine>(b, [&](auto* e) { return e->checkpoint_io(path, true); }) ? 0 : 1;
 }
 int lbfgsb_dev_checkpoint_read(lbfgsb_dev_t* h, const char* path) {
     EngineBase* b = (EngineBase*)h;
     if (!b || !path) return 1;
     g_last_error.clear();
-    return ((b->real_kind == 8) ? ((Engine<double>*)b)->checkpoint_io(path, false) : ((Engine<float>*)b)->checkpoint_io(path, false)) ? 0 : 1;
+    return with_kind<Engine>(b, [&](auto* e) { return e->checkpoint_io(path, false); }) ? 0 : 1;
 }
 
 int lbfgsb_minimize_dev_f64(lbfgsb_dev_t* h, double* x, const double* l, const double* u, const int32_t* nbd, lbfgsb_fg_dev_f64 fg,
@@ -2480,8 +2421,7 @@ int lbfgsb_minimize_graph_dev_f32(lbfgsb_dev_t* h, float* x, const float* l, con
 int lbfgsb_dev_graph_stats(lbfgsb_dev_t* h, int64_t* graph_steps, int64_t* launches_per_step) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return 1;
-    if (b->real_kind == 8) { Engine<double>* e = (Engine<double>*)b; *graph_steps = e->graph_steps; *launches_per_step = e->graph_launches_per_step; }
-    else { Engine<float>* e = (Engine<float>*)b; *graph_steps = e->graph_steps; *launches_per_step = e->graph_launches_per_step; }
+    with_kind<Engine>(b, [&](auto* e) { *graph_steps = e->graph_steps; *launches_per_step = e->graph_launches_per_step; });
     return 0;
 }
 
@@ -2504,26 +2444,25 @@ int lbfgsb_dev_active_set_hash(lbfgsb_dev_t* h, uint64_t* hash, int64_t* count) 
     EngineBase* b = (EngineBase*)h;
     if (!b) return 1;
     i64 c = 0;
-    bool ok = (b->real_kind == 8) ? ((Engine<double>*)b)->active_hash(hash, &c) : ((Engine<float>*)b)->active_hash(hash, &c);
+    bool ok = with_kind<Engine>(b, [&](auto* e) { return e->active_hash(hash, &c); });
     *count = c;
     return ok ? 0 : 1;
 }
 void* lbfgsb_dev_vector(lbfgsb_dev_t* h, int32_t which) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return nullptr;
-#define VSEL(E)                                                                                          \
-    switch (which) { case 0: return E->w.z; case 1: return E->w.r; case 2: return E->w.d; case 3: return E->w.t; \
-                     case 4: return E->w.xp; case 5: return E->w.ws; case 6: return E->w.wy; case 7: return E->w.iwhere; case 8: return E->w.gold; default: return nullptr; }
-    if (b->real_kind == 8) { Engine<double>* e = (Engine<double>*)b; VSEL(e) }
-    else { Engine<float>* e = (Engine<float>*)b; VSEL(e) }
+    return with_kind<Engine>(b, [&](auto* e) -> void* {
+        switch (which) { case 0: return e->w.z; case 1: return e->w.r; case 2: return e->w.d; case 3: return e->w.t;
+                         case 4: return e->w.xp; case 5: return e->w.ws; case 6: return e->w.wy; case 7: return e->w.iwhere; case 8: return e->w.gold; default: return nullptr; }
+    });
 }
 int lbfgsb_dev_vector_copy(lbfgsb_dev_t* h, int32_t which, void* dst_dev, int64_t bytes) {
     void* src = lbfgsb_dev_vector(h, which);
     if (!src || !dst_dev || bytes < 0) return 1;
     // never copy past the vector's allocation: m columns of ldw reals for ws / wy, ldw int32 for iwhere, ldw reals else
     EngineBase* b = (EngineBase*)h;
-    const i64 ldw = (b->real_kind == 8) ? ((Engine<double>*)b)->w.ldw : ((Engine<float>*)b)->w.ldw;
-    const i64 m = (b->real_kind == 8) ? ((Engine<double>*)b)->w.m : ((Engine<float>*)b)->w.m;
+    i64 ldw = 0, m = 0;
+    with_kind<Engine>(b, [&](auto* e) { ldw = e->w.ldw; m = e->w.m; });
     const i64 cap = (which == 7) ? ldw * 4 : ((which == 5 || which == 6) ? m : 1) * ldw * (i64)b->real_kind;
     if (bytes > cap) { set_error("lbfgsb_dev_vector_copy: %lld bytes requested, vector %d holds %lld", (long long)bytes, (int)which, (long long)cap); return 1; }
     if (cudaDeviceSynchronize() != cudaSuccess) return 1;
@@ -2532,57 +2471,54 @@ int lbfgsb_dev_vector_copy(lbfgsb_dev_t* h, int32_t which, void* dst_dev, int64_
 int lbfgsb_dev_exchange_mode(lbfgsb_dev_t* h) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return -1;
-    if (b->real_kind == 8) { Engine<double>* e = (Engine<double>*)b; return e->R <= 1 ? 0 : (e->p2p ? 2 : 1); }
-    Engine<float>* e = (Engine<float>*)b; return e->R <= 1 ? 0 : (e->p2p ? 2 : 1);
+    return with_kind<Engine>(b, [](auto* e) { return e->R <= 1 ? 0 : (e->p2p ? 2 : 1); });
 }
 int lbfgsb_dev_counters(lbfgsb_dev_t* h, int64_t* launches, int64_t* syncs) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return 1;
-    if (b->real_kind == 8) { *launches = ((Engine<double>*)b)->launches; *syncs = ((Engine<double>*)b)->syncs; }
-    else { *launches = ((Engine<float>*)b)->launches; *syncs = ((Engine<float>*)b)->syncs; }
+    with_kind<Engine>(b, [&](auto* e) { *launches = e->launches; *syncs = e->syncs; });
     return 0;
 }
 void lbfgsb_dev_profile(lbfgsb_dev_t* h, int32_t enable) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return;
-    if (b->real_kind == 8) ((Engine<double>*)b)->profile = enable != 0; else ((Engine<float>*)b)->profile = enable != 0;
+    with_kind<Engine>(b, [&](auto* e) { e->profile = enable != 0; });
 }
 void lbfgsb_dev_set_tie_limit(lbfgsb_dev_t* h, int64_t max_breakpoints) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return;
     i64 lim = max_breakpoints < 0 ? 0 : max_breakpoints;
-    if (b->real_kind == 8) { Engine<double>* e = (Engine<double>*)b; cudaStreamSynchronize(e->stream); cudaMemcpy(&e->s_dev->tie_limit, &lim, sizeof lim, cudaMemcpyHostToDevice); }
-    else { Engine<float>* e = (Engine<float>*)b; cudaStreamSynchronize(e->stream); cudaMemcpy(&e->s_dev->tie_limit, &lim, sizeof lim, cudaMemcpyHostToDevice); }
+    with_kind<Engine>(b, [&](auto* e) { cudaStreamSynchronize(e->stream); cudaMemcpy(&e->s_dev->tie_limit, &lim, sizeof lim, cudaMemcpyHostToDevice); });
 }
 int lbfgsb_dev_tie_stats(lbfgsb_dev_t* h, int64_t* replays, int64_t* not_replayed) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return 1;
     i64 ev = 0;
-    cudaError_t e;
-    if (b->real_kind == 8) { Engine<double>* g = (Engine<double>*)b; cudaStreamSynchronize(g->stream); e = cudaMemcpy(&ev, &g->s_dev->tie_events, sizeof ev, cudaMemcpyDeviceToHost); *replays = g->tie_replays; }
-    else { Engine<float>* g = (Engine<float>*)b; cudaStreamSynchronize(g->stream); e = cudaMemcpy(&ev, &g->s_dev->tie_events, sizeof ev, cudaMemcpyDeviceToHost); *replays = g->tie_replays; }
+    const cudaError_t ce = with_kind<Engine>(b, [&](auto* e) {
+        cudaStreamSynchronize(e->stream);
+        *replays = e->tie_replays;
+        return cudaMemcpy(&ev, &e->s_dev->tie_events, sizeof ev, cudaMemcpyDeviceToHost);
+    });
     *not_replayed = ev;
-    return e != cudaSuccess;
+    return ce != cudaSuccess;
 }
 void lbfgsb_dev_profile_reset(lbfgsb_dev_t* h) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return;
-    for (int q = 0; q < F_COUNT; ++q) {
-        if (b->real_kind == 8) { ((Engine<double>*)b)->fam_ms[q] = 0; ((Engine<double>*)b)->fam_calls[q] = 0; }
-        else { ((Engine<float>*)b)->fam_ms[q] = 0; ((Engine<float>*)b)->fam_calls[q] = 0; }
-    }
+    with_kind<Engine>(b, [](auto* e) { for (int q = 0; q < F_COUNT; ++q) { e->fam_ms[q] = 0; e->fam_calls[q] = 0; } });
 }
 int lbfgsb_dev_profile_read(lbfgsb_dev_t* h, int32_t cap, char* names, double* ms, double* bytes, int64_t* calls) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return 0;
-    int k = 0;
-    for (int q = 0; q < F_COUNT && k < cap; ++q, ++k) {
-        snprintf(names + 32 * k, 32, "%s", fam_name[q]);
-        if (b->real_kind == 8) { ms[k] = ((Engine<double>*)b)->fam_ms[q]; calls[k] = ((Engine<double>*)b)->fam_calls[q]; }
-        else { ms[k] = ((Engine<float>*)b)->fam_ms[q]; calls[k] = ((Engine<float>*)b)->fam_calls[q]; }
-        bytes[k] = 0;
-    }
-    return k;
+    return with_kind<Engine>(b, [&](auto* e) {
+        int k = 0;
+        for (int q = 0; q < F_COUNT && k < cap; ++q, ++k) {
+            snprintf(names + 32 * k, 32, "%s", fam_name[q]);
+            ms[k] = e->fam_ms[q]; calls[k] = e->fam_calls[q];
+            bytes[k] = 0;
+        }
+        return k;
+    });
 }
 
 int64_t lbfgsb_problem_scratch_bytes(void) { return (int64_t)sizeof(double) * (LBFGSB_GRID + 8); }
@@ -2607,13 +2543,9 @@ int lbfgsb_dev_trial_sums(lbfgsb_dev_t* h, lbfgsb_trial_sums_t* out) {
     EngineBase* b = (EngineBase*)h;
     if (!b || !out) return 1;
     memset(out, 0, sizeof *out);
-    if (b->real_kind == 8) {
-        Engine<double>* e = (Engine<double>*)b;
+    with_kind<Engine>(b, [&](auto* e) {
         out->d_dev = e->w.d; out->gd_part_dev = LB_SLOT(e->w.part, 0); out->pg_part_dev = LB_SLOT(e->w.part, 1); out->n = e->n;
-    } else {
-        Engine<float>* e = (Engine<float>*)b;
-        out->d_dev = e->w.d; out->gd_part_dev = LB_SLOT(e->w.part, 0); out->pg_part_dev = LB_SLOT(e->w.part, 1); out->n = e->n;
-    }
+    });
     out->grid = LBFGSB_GRID; out->block = LBFGSB_BLOCK; out->unroll = LBFGSB_UNROLL(b->real_kind); out->real_kind = b->real_kind;
     out->vec = LBFGSB_VEC(b->real_kind);
     return 0;
@@ -2621,8 +2553,7 @@ int lbfgsb_dev_trial_sums(lbfgsb_dev_t* h, lbfgsb_trial_sums_t* out) {
 void lbfgsb_dev_trial_sums_commit(lbfgsb_dev_t* h) {
     EngineBase* b = (EngineBase*)h;
     if (!b) return;
-    if (b->real_kind == 8) ((Engine<double>*)b)->trial_ready = true;   // consumed (or dropped) by the next setulb call
-    else ((Engine<float>*)b)->trial_ready = true;
+    with_kind<Engine>(b, [](auto* e) { e->trial_ready = true; });   // consumed (or dropped) by the next setulb call
 }
 int lbfgsb_problem_fused_f64(lbfgsb_dev_t* hh, int32_t kind, const double* x, double* g, const double* l, const double* u,
                              const int32_t* nbd, double* f_out, uint64_t seed) {
@@ -2801,20 +2732,14 @@ lbfgsb_batch_t* lbfgsb_batch_create(int32_t nprob, int64_t n, int32_t m, int32_t
     if (n > nmax) { set_error("lbfgsb_batch_create: n = %lld exceeds the one-CTA-per-problem limit of %lld variables", (long long)n, (long long)nmax); return nullptr; }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { set_error("no CUDA device (lbfgsb_b200 has no CPU path)"); return nullptr; }
-    if (real_kind == 8) {
-        BatchEngine<double>* e = new BatchEngine<double>();
-        if (!e->init(nprob, n, m, (cudaStream_t)cuda_stream)) { delete e; return nullptr; }
-        return (lbfgsb_batch_t*)e;
-    }
-    BatchEngine<float>* e = new BatchEngine<float>();
-    if (!e->init(nprob, n, m, (cudaStream_t)cuda_stream)) { delete e; return nullptr; }
-    return (lbfgsb_batch_t*)e;
+    if (real_kind == 8) return (lbfgsb_batch_t*)new_engine<BatchEngine<double>>(nprob, n, m, (cudaStream_t)cuda_stream);
+    return (lbfgsb_batch_t*)new_engine<BatchEngine<float>>(nprob, n, m, (cudaStream_t)cuda_stream);
 }
-void lbfgsb_batch_destroy(lbfgsb_batch_t* h) { delete (BatchBase*)h; }
+void lbfgsb_batch_destroy(lbfgsb_batch_t* h) { delete (HandleBase*)h; }
 void lbfgsb_batch_setulb_dev_f64(lbfgsb_batch_t* h, double* x, const double* l, const double* u, const int32_t* nbd, double* f_dev, double* g,
                                  const double* factr, const double* pgtol, char* task, char* csave, int32_t* lsave, int32_t* isave,
                                  double* dsave) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b || b->real_kind != 8) { set_error("invalid batch handle"); if (task) put60(task, "ERROR: INVALID LBFGSB_B200 HANDLE"); return; }
     BatchEngine<double>* e = (BatchEngine<double>*)b;
     if (!e->call(x, l, u, nbd, f_dev, g, *factr, *pgtol, task, csave, lsave, isave, dsave))
@@ -2823,7 +2748,7 @@ void lbfgsb_batch_setulb_dev_f64(lbfgsb_batch_t* h, double* x, const double* l, 
 void lbfgsb_batch_setulb_dev_f32(lbfgsb_batch_t* h, float* x, const float* l, const float* u, const int32_t* nbd, float* f_dev, float* g,
                                  const float* factr, const float* pgtol, char* task, char* csave, int32_t* lsave, int32_t* isave,
                                  float* dsave) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b || b->real_kind != 4) { set_error("invalid batch handle"); if (task) put60(task, "ERROR: INVALID LBFGSB_B200 HANDLE"); return; }
     BatchEngine<float>* e = (BatchEngine<float>*)b;
     if (!e->call(x, l, u, nbd, f_dev, g, *factr, *pgtol, task, csave, lsave, isave, dsave))
@@ -2840,43 +2765,40 @@ int lbfgsb_batch_minimize_graph_f32(lbfgsb_batch_t* h, float* x, const float* l,
     return batch_minimize_graph_impl<float>(h, x, l, u, nbd, f_dev, g, fg, user, factr, pgtol, max_iter, max_fg, task, csave, lsave, isave, dsave);
 }
 int lbfgsb_batch_graph_stats(lbfgsb_batch_t* h, int64_t* graph_builds, int64_t* graph_launches, int64_t* calls) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b || !graph_builds || !graph_launches || !calls) return 1;
-    if (b->real_kind == 8) { BatchEngine<double>* e = (BatchEngine<double>*)b; *graph_builds = e->graph_builds; *graph_launches = e->graph_launches; *calls = e->graph_calls; }
-    else { BatchEngine<float>* e = (BatchEngine<float>*)b; *graph_builds = e->graph_builds; *graph_launches = e->graph_launches; *calls = e->graph_calls; }
+    with_kind<BatchEngine>(b, [&](auto* e) { *graph_builds = e->graph_builds; *graph_launches = e->graph_launches; *calls = e->graph_calls; });
     return 0;
 }
 int lbfgsb_batch_counts(lbfgsb_batch_t* h, int32_t* n_fg, int32_t* n_newx, int32_t* n_done) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b) return 1;
-    if (b->real_kind == 8) { BatchEngine<double>* e = (BatchEngine<double>*)b; *n_fg = e->n_fg; *n_newx = e->n_newx; *n_done = e->n_done; }
-    else { BatchEngine<float>* e = (BatchEngine<float>*)b; *n_fg = e->n_fg; *n_newx = e->n_newx; *n_done = e->n_done; }
+    with_kind<BatchEngine>(b, [&](auto* e) { *n_fg = e->n_fg; *n_newx = e->n_newx; *n_done = e->n_done; });
     return 0;
 }
 void* lbfgsb_batch_fg_mask(lbfgsb_batch_t* h) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b) return nullptr;
-    return b->real_kind == 8 ? (void*)((BatchEngine<double>*)b)->bw.fgmask : (void*)((BatchEngine<float>*)b)->bw.fgmask;
+    return with_kind<BatchEngine>(b, [](auto* e) { return (void*)e->bw.fgmask; });
 }
 int lbfgsb_batch_get_iwhere(lbfgsb_batch_t* h, int32_t* iwhere_host) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b || !iwhere_host) return 1;
-    const int* src; i64 ldw, n; int nprob; cudaStream_t st;
-    if (b->real_kind == 8) { BatchEngine<double>* e = (BatchEngine<double>*)b; src = e->bw.iwhere; ldw = e->bw.ldw; n = e->bw.n; nprob = e->bw.nprob; st = e->stream; }
-    else { BatchEngine<float>* e = (BatchEngine<float>*)b; src = e->bw.iwhere; ldw = e->bw.ldw; n = e->bw.n; nprob = e->bw.nprob; st = e->stream; }
-    if (cudaMemcpy2DAsync(iwhere_host, (size_t)n * 4, src, (size_t)ldw * 4, (size_t)n * 4, (size_t)nprob, cudaMemcpyDeviceToHost, st) != cudaSuccess) return 1;
-    return cudaStreamSynchronize(st) != cudaSuccess;
+    return with_kind<BatchEngine>(b, [&](auto* e) {
+        const auto& bw = e->bw;
+        if (cudaMemcpy2DAsync(iwhere_host, (size_t)bw.n * 4, bw.iwhere, (size_t)bw.ldw * 4, (size_t)bw.n * 4, (size_t)bw.nprob, cudaMemcpyDeviceToHost, e->stream) != cudaSuccess) return 1;
+        return cudaStreamSynchronize(e->stream) != cudaSuccess ? 1 : 0;
+    });
 }
 int lbfgsb_batch_vector_copy(lbfgsb_batch_t* h, int32_t problem, int32_t which, void* dst_dev, int64_t bytes) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b || !dst_dev || bytes < 0) return 1;
-    if (b->real_kind == 8) return ((BatchEngine<double>*)b)->vector_copy(problem, which, dst_dev, bytes);
-    return ((BatchEngine<float>*)b)->vector_copy(problem, which, dst_dev, bytes);
+    return with_kind<BatchEngine>(b, [&](auto* e) { return e->vector_copy(problem, which, dst_dev, bytes); });
 }
 void* lbfgsb_batch_stream(lbfgsb_batch_t* h) {
-    BatchBase* b = (BatchBase*)h;
+    HandleBase* b = (HandleBase*)h;
     if (!b) return nullptr;
-    return b->real_kind == 8 ? (void*)((BatchEngine<double>*)b)->stream : (void*)((BatchEngine<float>*)b)->stream;
+    return with_kind<BatchEngine>(b, [](auto* e) { return (void*)e->stream; });
 }
 int lbfgsb_problem_rosenbrock_batch_f64(int32_t nprob, int64_t n, const double* x_dev, double* g_dev, double* f_dev, const int32_t* mask_dev,
                                         void* st) {
